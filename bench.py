@@ -3,6 +3,7 @@
 bench.py — benchmark of the read -> feature -> count path on every workload BASELINE.json names.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--reads R] [--configs a,b,...] [--scale S]
+                    [--dump-outputs DIR]
 
 Headline (the JSON line's own metric/value/e2e/roofline, comparable across rounds): BASELINE.json configs[1],
 synthetic 100 M x 50 bp reads per GPU vs a 2 000-guide library, --st 0 --l 20 --m 1 --ph 30; weak scaling over GPUs.
@@ -139,6 +140,53 @@ def committed_traffic():
         return None
 
 
+DUMP_LIMIT = 64 << 20                # bytes of all arrays --dump-outputs writes
+DUMP_ARRAY_ELEMS = 1 << 21           # a larger array keeps a fixed, seeded sample of its rows
+
+
+class OutputDump:
+    """--dump-outputs DIR: what the last timed step of each leg handed to its caller, as DIR/<name>.npy, so that two builds
+    can be compared output for output (the inputs are seeded: the same arguments give the same inputs).  Counts and
+    statistics are float64, exact below 2**53; an array of more than DUMP_ARRAY_ELEMS elements keeps the rows of a fixed,
+    seeded sample, in their original order."""
+
+    def __init__(self, path):
+        self.dir, self.nbytes = path, 0
+        os.makedirs(path, exist_ok=True)
+
+    @staticmethod
+    def rows(n, row_elems):
+        keep = max(1, DUMP_ARRAY_ELEMS // max(1, row_elems))
+        if n <= keep:
+            return np.arange(n)
+        return np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+
+    def save(self, name, a):
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > DUMP_ARRAY_ELEMS:
+            a = a[self.rows(a.shape[0], a.size // a.shape[0])]
+        if self.nbytes + a.nbytes > DUMP_LIMIT:
+            raise RuntimeError(f"--dump-outputs: {name} would take the dump past {DUMP_LIMIT >> 20} MB")
+        self.nbytes += a.nbytes
+        np.save(os.path.join(self.dir, name + ".npy"), a)
+
+    def save_stats(self, name, stats):
+        """one stats dict (or a list of them, one per sample) in STAT_NAMES order"""
+        self.save(name, [list(s.values()) for s in stats] if isinstance(stats, list) else list(stats.values()))
+
+    def save_table(self, name, table):
+        """an Extract+Count key table: one row per key in byte order — count, key length, the key's bytes (0-padded)"""
+        keys = sorted(table)
+        width = max((len(k) for k in keys), default=0)
+        idx = self.rows(len(keys), 2 + width)
+        a = np.zeros((len(idx), 2 + width))
+        for r, i in enumerate(idx):
+            k = keys[i]
+            a[r, 0], a[r, 1] = table[k], len(k)
+            a[r, 2:2 + len(k)] = np.frombuffer(k, dtype=np.uint8)
+        self.save(name, a)
+
+
 def library():
     synth = importlib.import_module("2fast2q_b200.synth")        # generator spec + library builder (not the oracle)
     return synth.make_library(CONFIG, N_GUIDES, FEAT_LEN), synth.default_spec(CONFIG)
@@ -148,13 +196,13 @@ def library():
 # the reference arm
 # ------------------------------------------------------------------------------------------------------------
 def real_reference(keys, names, spec, reads, cores, timeout_s=240):
-    """the UNMODIFIED Python reference (baseline/_ref, copied from /root/reference by build()) through its own CLI on a
+    """the UNMODIFIED Python reference (its fast2q package placed by hand in the git-ignored baseline/_ref) through its own CLI on a
     slice of the config-2 stream written as `cores` files (file-parallel = its best case, SURVEY.md §8d)"""
     import shutil
     import tempfile
     ref = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref, "fast2q")):
-        return {"unavailable": "baseline/_ref/fast2q is absent (build() copies it where /root/reference exists)"}
+        return {"unavailable": "baseline/_ref/fast2q is absent (place the unmodified reference package there)"}
     synth = importlib.import_module("2fast2q_b200.synth")
     tmp = tempfile.mkdtemp(prefix="f2q_ref_")
     try:
@@ -165,7 +213,8 @@ def real_reference(keys, names, spec, reads, cores, timeout_s=240):
             synth.fixed_reads(keys, t * per, per, **spec).tofile(os.path.join(src, "s%03d.fastq" % t))
         with open(os.path.join(tmp, "lib.csv"), "w") as f:
             f.write("".join(f"{n},{k.decode()}\n" for n, k in zip(names, keys)))
-        env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ref, "_stubs"), ref]), PYTHONWARNINGS="ignore",
+        stubs = os.path.join(ROOT, "tests", "golden", "_stubs")                # colorama / matplotlib, cosmetic on the counting path
+        env = dict(os.environ, PYTHONPATH=os.pathsep.join([stubs, ref]), PYTHONWARNINGS="ignore",
                    NUMBA_CACHE_DIR=os.path.join(tmp, "nc"))
         cmd = [sys.executable, "-m", "fast2q", "-c", "--s", src, "--g", os.path.join(tmp, "lib.csv"), "--o", out, "--pb",
                "--cp", str(cores), "--m", "1", "--ph", "30", "--st", "0", "--l", str(FEAT_LEN)]
@@ -451,6 +500,7 @@ def run_workload(w, env):
             gen(s * w.reads, w.reads, at=k * w.reads * rec)                   # every sample owns its own read range
         resident_once = True
     pin_res = [lib.PinnedBuffer(8 * (n_keys + 6)) for _ in range(max(1, len(my_samples) if w.n_samples > 1 else 1))]
+    ec_stats = {}
 
     def resident_pass(limit=None):
         """returns device ms of the pass (synth of per-chunk generated workloads excluded)"""
@@ -484,7 +534,7 @@ def run_workload(w, env):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(stream)
             merge_counts()
-            eng.end()
+            ec_stats.update(eng.end()[1])
             merge_ec()
             e1.record(stream)
             evs.append((e0, e1))
@@ -494,7 +544,7 @@ def run_workload(w, env):
     for _ in range(3):                                                        # warm-up
         resident_pass(limit=min(2, len(chunks)) if w.n_samples == 1 else None)
     barrier()
-    n_pass = 1 if (w.n_samples == 1 and len(chunks) > 4) else 3
+    n_pass = env["args"].steps
     l0 = eng.launches
     t_w0 = time.perf_counter()
     ms_res = sum(resident_pass() for _ in range(n_pass)) / n_pass
@@ -505,6 +555,17 @@ def run_workload(w, env):
         c_k, s_k = eng.read_async_result(pin_res[-1] if w.n_samples > 1 else pin_res[0])
         exp_reads = w.reads if w.n_samples > 1 else total_reads
         assert s_k["reads"] == exp_reads, (w.name, s_k, exp_reads)
+    dump = env["dump"]
+    if dump and w.ec:
+        dump.save_table(w.name + "_table", eng.ec_items())
+        dump.save_stats(w.name + "_stats", ec_stats)
+    elif dump and w.n_samples > 1:
+        res = [eng.read_async_result(b) for b in pin_res]                   # this rank's samples
+        dump.save(w.name + "_counts", [c for c, _ in res])
+        dump.save_stats(w.name + "_stats", [s for _, s in res])
+    elif dump:
+        dump.save(w.name + "_counts", c_k)
+        dump.save_stats(w.name + "_stats", s_k)
     t = torch.tensor([ms_res], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -546,12 +607,13 @@ def run_workload(w, env):
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         tw = time.perf_counter()
         f0.record(stream)
-        done = e2e_pass()
+        for _ in range(n_pass):
+            done = e2e_pass()
         f1.record(stream)
         barrier()
         env["windows"].append((tw, time.perf_counter()))
-        wall = (time.perf_counter() - tw) * 1e3
-        ms2 = f0.elapsed_time(f1)
+        wall = (time.perf_counter() - tw) * 1e3 / n_pass
+        ms2 = f0.elapsed_time(f1) / n_pass
         t = torch.tensor([ms2, wall, float(done)], dtype=torch.float64, device=dev)
         if world > 1:
             tm = t.clone()
@@ -624,6 +686,7 @@ def run_gpu(args, rank, local_rank, world):
         comm_eng.comm_init_rank(box[0], world, rank)
     clocks = ClockSampler(local_rank, gpu_uuid)
     windows = []
+    dump = OutputDump(args.dump_outputs) if args.dump_outputs and rank == 0 else None
     out = None
 
     def barrier():
@@ -686,6 +749,9 @@ def run_gpu(args, rank, local_rank, world):
             c_k, s_k = eng.read_async_result(b)
             assert s_k == stats and np.array_equal(c_k, counts), "a timed pass returned different counts"
             b.free()
+        if dump:
+            dump.save("headline_counts", c_k)
+            dump.save_stats("headline_stats", s_k)
         launches = eng.launches - l0
         ms = e0.elapsed_time(e1) / args.steps
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -722,12 +788,15 @@ def run_gpu(args, rank, local_rank, world):
             t0 = time.perf_counter()
             f0.record(stream)
             for _ in range(args.steps):
-                step_e2e()
+                c2, s2 = step_e2e()
             f1.record(stream)
             barrier()
             windows.append((t0, time.perf_counter()))
             wall = (time.perf_counter() - t0) / args.steps * 1e3
             ms2 = max(f0.elapsed_time(f1) / args.steps, 0.0)
+            if dump:
+                dump.save("headline_e2e_counts", c2)
+                dump.save_stats("headline_e2e_stats", s2)
             t = torch.tensor([ms2, wall], dtype=torch.float64, device=dev)
             if world > 1:
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -785,7 +854,7 @@ def run_gpu(args, rank, local_rank, world):
     others = {}
     if want - {"headline"}:
         env = dict(lib=lib, multi=multi, host=host_mod, rank=rank, world=world, dev=dev, stream=stream, local_rank=local_rank,
-                   args=args, windows=windows, comm=comm_eng)
+                   args=args, windows=windows, comm=comm_eng, dump=dump)
         for name, w in build_workloads(args).items():
             t0 = time.perf_counter()
             r = run_workload(w, env)
@@ -882,6 +951,7 @@ def main():
     ap.add_argument("--pinned", default="default", choices=["default", "wc"], help="pinned host memory of the end-to-end leg: default | write-combined")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each leg returned as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)

@@ -1,19 +1,18 @@
 #!/usr/bin/env python
 """
 Golden fixtures for the drop-in surface (CLI, features .csv loader, *_reads.csv / compiled.csv /
-compiled_stats.csv): runs the UNMODIFIED reference CLI (`python -m fast2q -c ...` from /root/reference, with the
-colorama / matplotlib stubs of tests/golden/_stubs) on small input folders and stores inputs + outputs in
-tests/golden/cli_cases.json.gz.  Build container only:
+compiled_stats.csv): runs the UNMODIFIED reference CLI (`python -m fast2q -c ...` from the checkout refharness.py
+points at, with the colorama / matplotlib stubs of tests/golden/_stubs) on the input folders of tests/cli_golden.py
+and stores its outputs in tests/golden/cli_cases.json.gz with what tests/cli_golden.py needs to regenerate and check
+the inputs (cli_golden.file_entry).  Needs the reference checkout:
 
     python tests/golden/make_cli_golden.py
 
 Also stores the reference's features_loader() result for a few awkward library files and the reference's
 input_parser() dict for a few command lines.
 """
-import base64
 import glob
 import gzip
-import io
 import json
 import os
 import subprocess
@@ -24,69 +23,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, HERE)
 sys.path.insert(0, ROOT)
-import cases  # noqa: E402
+sys.path.insert(0, os.path.dirname(HERE))
+import cli_golden  # noqa: E402
 import refharness  # noqa: E402
-from oracle import synth  # noqa: E402
-
-
-def gz(data: bytes, level=6) -> bytes:
-    b = io.BytesIO()
-    with gzip.GzipFile(fileobj=b, mode="wb", compresslevel=level, mtime=0) as f:
-        f.write(data)
-    return b.getvalue()
-
-
-def cli_cases():
-    out = []
-    # 1. Counter, fixed position, three files (.fastq, .fastq.gz, CRLF .fastq), numeric names, awkward library file
-    names, keys = synth.make_library(2, 150, 20)
-    spec = synth.default_spec(2)
-    lib_lines = []
-    for i, k in enumerate(keys):
-        s = k.decode()
-        if i == 7:
-            s = s.lower()
-        if i == 9:
-            s = s[:10] + " " + s[10:]
-        lib_lines.append(f"{i + 1},{s}")
-    lib_lines.insert(20, f"999,{keys[3].decode()}")            # shares its sequence with entry 4: ignored with a warning
-    # (a repeated NAME makes the reference itself crash in run_stats, fast2q.py:1475, so none is used here)
-    reads = synth.fixed_reads(keys, 0, 5400, **spec).tobytes()
-    rec = 118
-    c = reads[5000 * rec:5400 * rec].replace(b"\n", b"\r\n")
-    out.append(dict(name="cli_counter", library="\n".join(lib_lines) + "\n",
-                    files={"sampleA.fastq": reads[:3000 * rec], "sampleB.fastq.gz": gz(reads[3000 * rec:5000 * rec]),
-                           "sampleC.fastq": c},
-                    args=["--m", "1", "--ph", "30", "--k", "--pb", "--cp", "2"]))
-    # 2. Extract + Count between delimiters with mismatches, two files
-    bs = synth.barseq_reads(4, 3000)
-    cut = bs.find(b"\n@", len(bs) // 2) + 1
-    out.append(dict(name="cli_ec", library=None, files={"bar1.fastq": bs[:cut], "bar2.fastq.gz": gz(bs[cut:])},
-                    args=["--mo", "EC", "--us", "GTTCAGAGTTCT", "--ds", "CTGAATAGGCCA", "--msu", "1", "--msd", "1", "--pb", "--k",
-                          "--cp", "2"]))
-    # 3. dual fixed windows, ';' separated library, alphabetical names, custom file name, intermediates deleted
-    dn, dk, xs, ys = synth.dual_library(5, 120)
-    dr = synth.dual_reads(5, 2400, xs, ys, mode="fixed")
-    cut = dr.find(b"\n@", len(dr) // 3) + 1
-    out.append(dict(name="cli_dual", library="".join(f"{n};{k.decode()}\n" for n, k in zip(dn, dk)),
-                    files={"d_one.fastq": dr[:cut], "d_two.fastq": dr[cut:]},
-                    args=["--st", "0,30", "--l", "20", "--m", "1", "--pb", "--cp", "2", "--fn", "mycounts"]))
-    # 4. a single file: File-Split mode is forced (fast2q.py:1671-1672); --cp 1 keeps the reference's chunking exact
-    out.append(dict(name="cli_single_split", library="".join(f"{n},{k.decode()}\n" for n, k in zip(names, keys)),
-                    files={"only.fastq.gz": gz(reads[:2000 * rec])}, args=["--m", "2", "--pb", "--k", "--cp", "1"]))
-    # 5. a gzip file cut off mid-stream: warning + partial counts (fast2q.py:405-407)
-    whole = gz(reads[:2500 * rec])
-    out.append(dict(name="cli_truncated_gz", library="".join(f"{n},{k.decode()}\n" for n, k in zip(names, keys)),
-                    files={"good.fastq": reads[2500 * rec:3500 * rec], "cut.fastq.gz": whole[: len(whole) * 6 // 10]},
-                    args=["--pb", "--k", "--cp", "2"]))
-    # 6. delimiter pairs in Counter mode, tab separated library
-    n5, k5, xs5, ys5 = synth.dual_library(5, 100)
-    d5 = synth.dual_reads(5, 1500, xs5, ys5, mode="delim")
-    cut = d5.find(b"\n@", len(d5) // 2) + 1
-    out.append(dict(name="cli_dual_delim", library="".join(f"{n}\t{k.decode()}\n" for n, k in zip(n5, k5)),
-                    files={"p1.fastq": d5[:cut], "p2.fastq": d5[cut:]},
-                    args=["--us", "ACCGGT,GGATCC", "--ds", "TTGACA,CAATTG", "--m", "1", "--pb", "--k", "--cp", "2"]))
-    return out
 
 
 def run_reference_cli(case):
@@ -145,10 +84,10 @@ def main():
     assert refharness.available()
     ref = refharness.load()
     out = dict(cli=[], loader={}, parser=[])
-    for c in cli_cases():
+    for c in cli_golden.cli_inputs():
         outs, stdout = run_reference_cli(c)
         out["cli"].append(dict(name=c["name"], args=c["args"], library=c["library"],
-                               files={k: base64.b64encode(v).decode() for k, v in c["files"].items()}, outputs=outs))
+                               files={k: cli_golden.file_entry(k, v) for k, v in c["files"].items()}, outputs=outs))
         print(c["name"], {k: len(v) for k, v in outs.items()})
     for name, text in loader_cases().items():
         with tempfile.NamedTemporaryFile("w", suffix=".csv", delete=False) as f:
