@@ -95,7 +95,10 @@ SYMBOLS = {
     "f2q_kernel_times": (C.c_int, [_VP, C.POINTER(C.c_double), _U64P]),
     "f2q_spec_counts": (C.c_int, [_VP, _U64P, _U64P]),
     "f2q_memo_counts": (C.c_int, [_VP, _U64P, _U64P]),
+    "f2q_get_info": (C.c_int, [_VP, C.c_char_p, C.POINTER(C.c_int64)]),
 }
+POLICIES = ("generic", "fast1", "flex_S", "flex_B")          # f2q_get_info "policy"
+TABLES = ("probing", "compact", "cuckoo", "cuckoo+neighbours")   # f2q_get_info "table"
 
 _lib = None
 
@@ -455,6 +458,17 @@ class Engine:
         a, b = C.c_uint64(), C.c_uint64()
         self._ck(self.L.f2q_memo_counts(self.h, C.byref(a), C.byref(b)))
         return int(a.value), int(b.value)
+
+    def info(self, name: str):
+        """f2q_get_info: which table / policy / plan the context chose.  "policy" and "table" come back as the names of
+        POLICIES / TABLES, everything else as an int"""
+        v = C.c_int64()
+        self._ck(self.L.f2q_get_info(self.h, name.encode(), C.byref(v)))
+        if name == "policy":
+            return POLICIES[v.value]
+        if name == "table":
+            return TABLES[v.value]
+        return int(v.value)
 
     def kernel_times(self):
         """{'tile': (ms, launches), 'resolve': ..., 'generic': ..., 'aux': ...} of the last finished sample (option time_kernels)"""

@@ -154,6 +154,7 @@ struct f2q_ctx {
     bool slow_valid = false;
     bool async_pending = false;        // f2q_end_sample_async results not yet waited for (kernel timings are collected by f2q_sync)
     uint64_t spec_counts[2] = {0, 0};  // last finished sample: chunks committed by the speculation / parsed by the exact kernel
+    int hist_used = 0;                 // this sample: launched with the shared-memory histogram, bit 0 the streaming kernel, bit 1 the exact kernel
     int nt = 256;                      // threads (= owned rows) per tile-kernel CTA: 256 for the packed policy (measured 35 % faster),
     bool nt_user = false;              // 128 for the generic per-read code, unless option "tile_threads" says otherwise
     // optional per-kernel timing (option "time_kernels"): event pairs around the tile / resolver / generic launches
@@ -292,6 +293,7 @@ template <int POLICY, int CH, int NT>
 int launch_tile(f2q_ctx* c, const TileParams& P, Outputs O, uint64_t n_tiles_upper) {
     const bool hist = (POLICY == POLICY_FAST1) && c->n_keys > 0 && c->n_keys <= HIST_MAX_KEYS;
     TileParams p = P; p.hist_smem = hist;
+    if (hist) c->hist_used |= 2;
     const size_t smem = tile_smem_bytes<CH, NT>(hist ? c->n_keys : 0);
     unsigned grid = 0;
     int rc = tile_grid<POLICY, CH, NT>(c, &grid); if (rc) return rc;
@@ -344,6 +346,7 @@ int launch_spec(f2q_ctx* c, const SpecParams& P, Outputs O) {
         CU(c, cudaFuncSetAttribute(k_spec<POLICY, CH, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SM_SMEM_BYTES - sizeof(GenericCfg) - SPEC_SMEM_MARGIN)));
         ready = 1;
     }
+    if (hist) c->hist_used |= 1;
     k_spec<POLICY, CH, W><<<(unsigned)c->sm_count, W * 32, smem, c->stream>>>(p, c->dG, c->T, c->E, O, reinterpret_cast<const SlowArgs*>(c->slow_args.p) + 1, c->hG.flex);
     c->launches++;
     CU(c, cudaGetLastError());
@@ -1305,6 +1308,7 @@ F2Q_EXPORT int f2q_begin_sample(f2q_ctx* c) {
     if ((rc = dev_alloc(c, c->carry, c->carry_cap + 256))) return rc;
     if ((rc = dev_alloc(c, c->status_stitch, c->carry_cap / (64 * 16 * 3) + 2 + 64))) return rc;
     if (!c->ch_from_device) c->ch_decided = false;
+    c->hist_used = 0;
     {
         const uint64_t nw = (uint64_t)c->n_keys + 5;
         k_begin<<<(unsigned)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c->sm_count), 256, 0, c->stream>>>(
@@ -2400,6 +2404,25 @@ F2Q_EXPORT uint64_t f2q_launch_count(const f2q_ctx* c) { return c ? c->launches 
 F2Q_EXPORT int f2q_spec_counts(const f2q_ctx* c, uint64_t* committed, uint64_t* fell_back) {
     if (!c || !committed || !fell_back) return F2Q_EINVAL;
     *committed = c->spec_counts[0]; *fell_back = c->spec_counts[1];
+    return F2Q_OK;
+}
+
+F2Q_EXPORT int f2q_get_info(f2q_ctx* c, const char* name, int64_t* value) {
+    int rc = check_ctx(c); if (rc) return rc;
+    if (!name || !value) return fail(c, F2Q_EINVAL, "null argument");
+    const std::string n(name);
+    if (n == "policy") *value = c->policy;
+    else if (n == "table") *value = c->T.cuckoo ? (c->T.ck_neighbours ? 3 : 2) : c->T.cslots ? 1 : 0;
+    else if (n == "hist") *value = c->hist_used;
+    else if (n == "seed_parts") *value = c->T.seed_ncombo ? (int64_t)c->T.seed_parts : 0;
+    else if (n == "flex_table") *value = c->T.fx_slots ? 1 : 0;
+    else if (n == "generic_reads") {
+        if (c->in_sample) return fail(c, F2Q_ESTATE, "generic_reads is known once the sample has finished");
+        unsigned long long v = 0;
+        CU(c, cudaStreamSynchronize(c->stream));
+        CU(c, cudaMemcpy(&v, &c->dS->generic_reads, sizeof(v), cudaMemcpyDeviceToHost));
+        *value = (int64_t)v;
+    } else return fail(c, F2Q_EINVAL, "unknown info " + n);
     return F2Q_OK;
 }
 

@@ -137,6 +137,7 @@ struct DevState {
     uint32_t spec_off;             // sticky per sample: a speculation failed, later chunks go straight to the exact kernel
     uint32_t spec_commits, spec_fallbacks;   // chunks of this sample whose speculation held / that the exact kernel parsed
     unsigned long long memo_lookups, memo_hits;
+    unsigned long long generic_reads;   // reads the generic read queue took this sample (k_generic_queue, f2q_get_info)
     unsigned long long dbg[8];     // diagnostics (F2Q_DEBUG=1): failed mbarrier tries per wait site, look-back rounds / spins
 };
 

@@ -321,15 +321,16 @@ __device__ __forceinline__ int g_rstrip(const uint8_t* p, int n) {
     return n;
 }
 
-// drains the generic read queue: one thread per entry
+// drains the generic read queue: one thread per entry (and one thread of the launch adds the fill to S->generic_reads)
 __global__ void __launch_bounds__(128) k_generic_queue(const GenericCfg* __restrict__ Gp, const SlowArgs* __restrict__ X,
-                                                       const GEntry* q, const DevState* S) {
+                                                       const GEntry* q, DevState* S) {
     __shared__ GenericCfg G;
     for (uint32_t i = threadIdx.x; i < sizeof(GenericCfg) / 4; i += blockDim.x)
         reinterpret_cast<uint32_t*>(&G)[i] = reinterpret_cast<const uint32_t*>(Gp)[i];
     __syncthreads();
     unsigned long long st[F2Q_N_STATS] = {0, 0, 0, 0, 0};
     uint32_t n = S->g_count < S->g_cap ? S->g_count : S->g_cap;
+    if (blockIdx.x == 0 && threadIdx.x == 0) S->generic_reads += n;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         GEntry e = q[i];
         const uint8_t* R = reinterpret_cast<const uint8_t*>(e.seq_addr);

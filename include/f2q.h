@@ -300,6 +300,21 @@ int f2q_spec_counts(const f2q_ctx* ctx, uint64_t* committed, uint64_t* fell_back
  * lives with the library — across chunks and samples of the context — and never changes a count (option "memo_entries"). */
 int f2q_memo_counts(const f2q_ctx* ctx, uint64_t* lookups, uint64_t* hits);
 
+/* read-only view of the shapes the context chose, by name (results never depend on them; tests use them to prove which
+ * side of a size threshold an input landed on):
+ *   "policy"        per-read code of the streaming kernel: 0 byte-wise generic | 1 fast1 (one fixed window, Counter) |
+ *                   2 flex_S (bit-parallel, 96-position planes, k <= 1) | 3 flex_B (160-position planes, k <= 3).
+ *                   Final after the first submit of a sample (the record length sniffed there can move flex_S to flex_B)
+ *   "table"         exact lookup table of the packed library keys: 0 probing | 1 compact | 2 two-choice cuckoo |
+ *                   3 cuckoo that also holds every Hamming-1 neighbour
+ *   "hist"          this sample's launches used the per-CTA shared-memory histogram: bit 0 the streaming kernel, bit 1 the
+ *                   exact kernel
+ *   "seed_parts"    segments P of the resolver's seed plan; 0 = the classic m + 1 one-segment seeds (or no seed index)
+ *   "flex_table"    1 when the library has the flex tables (every key <= 2 ACGT pieces of <= 32 symbols)
+ *   "generic_reads" reads the generic read queue took during the last finished sample (one device-to-host copy per call;
+ *                   F2Q_ESTATE inside a sample) */
+int f2q_get_info(f2q_ctx* ctx, const char* name, int64_t* value);
+
 /* device time of the last finished sample per kernel class, measured with CUDA events on the context's stream
  * (needs option "time_kernels" = 1): [0] fused tile kernel over the chunk (the streaming kernel when "spec" is on),
  * [1] mismatch resolver, [2] generic queue, [3] speculation verify + commit + the exact kernel behind it (which

@@ -114,3 +114,81 @@ def test_ineligible_configurations_are_refused():
     for kw in (dict(upstream="ACGN"), dict(upstream="ACGT", miss_search_up=4), dict(start="0,1,2"), dict(upstream="A" * 33),
                dict(start="0", length=33)):
         assert H.hc_flex_eligible(C.byref(lib.make_config(**kw))) == 0, kw
+
+
+# the 160-position planes of flex_B (PW = 5): flex_pieces (flex_core.h) loads 8 * (4 PW - 2) = 144 positions when the warp's
+# longest line allows it and all 160 otherwise (PW = 3: 80 / 96).  Reads of 81..160 positions, pieces of 29..33 symbols
+# around the 32-symbol piece limit (FLEX_MAX_PIECE), each read also run as if the warp's longest line sat on either side of
+# the 80/81 and 144/145 group boundaries
+LONG_CONFIGS = [
+    dict(mode="EC", upstream="GTTCAGAGTTCT", downstream="CTGAATAGGCCA", miss_search_up=1, miss_search_down=1),
+    dict(mode="EC", upstream="GTTCAGAGTTCT", downstream="CTGAATAGGCCA", miss_search_up=3, miss_search_down=2),
+    dict(mode="EC", upstream="ACGTTGCAACGTTGCAACGTTGCAACGTTGCA", miss_search_up=3, length=31),
+    dict(mode="EC", downstream="G", miss_search_down=0, length=32),
+    dict(mode="C", upstream="ACCGGT,GGATCC", downstream="TTGACA,CAATTG", miss_search_up=1, miss_search_down=1),
+]
+LONG_LENGTHS = [81, 82, 95, 96, 97, 120, 143, 144, 145, 146, 159, 160]
+
+
+def long_reads(seed, n, kw):
+    r = synth.SM64(seed)
+    ups = (kw.get("upstream") or "").split(",")
+    downs = (kw.get("downstream") or "").split(",")
+    for _ in range(n):
+        target = r.choice(LONG_LENGTHS) if r.below(2) else 81 + r.below(80)
+        s = bytearray(r.dna(r.below(40)))
+        for i in range(max(len(ups), len(downs))):
+            u = ups[i % len(ups)].encode() if ups[0] else b""
+            d = downs[i % len(downs)].encode() if downs[0] else b""
+            if u and r.below(100) < 30:
+                u = synth.mutate(r, u, 1 + r.below(4))
+            if d and r.below(100) < 30:
+                d = synth.mutate(r, d, 1 + r.below(3))
+            s += u + r.dna(29 + r.below(5)) + d
+        s = bytes(s + r.dna(max(0, target - len(s))))[:target]
+        t = r.below(100)
+        if t < 8:
+            p = r.below(len(s))
+            s = s[:p] + r.choice([b"N", b"n", b"a", b"\xc1"] + ([b":"] if len(ups) == len(downs) == 1 else [])) + s[p + 1:]
+        q = bytearray(63 + r.below(11) for _ in range(len(s)))
+        if r.below(100) < 15:
+            q[r.below(len(q))] = r.choice([33, 40, 52, 61])
+        q = bytes(q)
+        t = r.below(100)
+        if t < 6:
+            q = q[: r.below(len(q) + 1)]
+        elif t < 12:
+            q = (q + bytes(63 + r.below(11) for _ in range(1 + r.below(20))))[:160]     # quality line longer than the sequence line
+        yield s, q
+
+
+@pytest.mark.parametrize("k", range(len(LONG_CONFIGS)))
+def test_flex_extraction_of_reads_longer_than_96_positions(k, oracle):
+    kw = LONG_CONFIGS[k]
+    cfg = lib.make_config(**kw)
+    ocfg = oracle.make_config(**kw)
+    n_keys = n_long_piece = 0
+    sides = set()
+    for s, q in long_reads(2000 + k, 2500, kw):
+        want = oracle.build_key(ocfg, s, q)
+        m = max(len(s), len(q))
+        # the warp's longest line: this read's own, and either side of the group boundaries it can still reach
+        for maxlen in sorted({m} | {b for b in (80, 81, 144, 145, 160) if b >= m}):
+            sides.add(maxlen <= 144)                            # narrow plane load (flex_pieces: maxlen <= 8 * (4 PW - 2))
+            rc, got = flex_key(cfg, 5, s, q, maxlen - m)
+            assert rc != -3, (kw, s, q)
+            if rc == -2:
+                assert want is not None, (kw, s, q)
+                pieces = want.split(b":") if cfg.n_iter > 1 else [want]     # (a single piece may hold a ':' of the read)
+                assert max(len(p) for p in pieces) > 32, (kw, s, q, want)
+                n_long_piece += 1
+                continue
+            if want is None:
+                assert rc == -1, (kw, s, q, got)
+            else:
+                assert rc >= 0 and got == want, (kw, maxlen, s, q, got, want)
+                n_keys += 1
+    assert n_keys > 500, n_keys
+    assert sides == {True, False}
+    if kw.get("upstream") and kw.get("downstream"):
+        assert n_long_piece > 10, n_long_piece                  # 33-symbol pieces reached the generic hand-over
