@@ -63,6 +63,7 @@ SYMBOLS = {
     "f2q_set_library": (C.c_int, [_VP, _VP, _VP, C.c_uint32]),
     "f2q_begin_sample": (C.c_int, [_VP]),
     "f2q_submit": (C.c_int, [_VP, _VP, C.c_uint64, C.c_int]),
+    "f2q_submit_file_sharded": (C.c_int, [C.POINTER(_VP), C.c_int, C.c_char_p, C.c_int, _U64P, C.c_int, _I32P, _U64P]),
     "f2q_submit_device": (C.c_int, [_VP, _VP, C.c_uint64, C.c_int]),
     "f2q_submit_file": (C.c_int, [_VP, C.c_char_p, C.c_int, C.c_uint64, C.c_int, _I32P, _U64P]),
     "f2q_sync": (C.c_int, [_VP]),
@@ -233,6 +234,20 @@ def allreduce_counts(engines):
 def ec_merge(engines):
     arr = (C.c_void_p * len(engines))(*[e.h for e in engines])
     engines[0]._ck(load().f2q_ec_merge(arr, len(engines)))
+
+
+def submit_file_sharded(engines, path, is_gzip, cuts=None, threads=8):
+    """one plain or bgzip file as one sample parsed by every engine (each inside a freshly begun sample; f2q_submit_file_sharded).
+    engines[0] then holds the whole sample (end() / ec_items() on it), the others are closed and empty.  cuts: None (even
+    ranges of >= 64 MiB) or len(engines) - 1 file offsets.  Returns (complete, uncompressed bytes) as Engine.submit_file."""
+    arr = (C.c_void_p * len(engines))(*[e.h for e in engines])
+    cut_arr = (C.c_uint64 * max(1, len(engines) - 1))(*[int(x) for x in cuts]) if cuts is not None else None
+    if cuts is not None and len(cuts) != len(engines) - 1:
+        raise ValueError("cuts needs one offset fewer than there are engines")
+    ok, nb = C.c_int32(1), C.c_uint64(0)
+    engines[0]._ck(load().f2q_submit_file_sharded(arr, len(engines), os.fsencode(path), int(bool(is_gzip)), cut_arr, int(threads),
+                                                  C.byref(ok), C.byref(nb)))
+    return bool(ok.value), int(nb.value)
 
 
 class PinnedBuffer:

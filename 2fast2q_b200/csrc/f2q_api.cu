@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <chrono>
@@ -133,6 +134,13 @@ struct f2q_ctx {
     size_t q_entry = 0;                              // bytes per entry the queue buffer was sized for
     int64_t opt_generic_entries = 0;
     std::vector<uint64_t> ec_drain_off, ec_drain_cnt; std::vector<uint8_t> ec_drain_keys; bool ec_drained = false;
+    // one file on several contexts (f2q_submit_file_sharded)
+    uint64_t lib_hash = 0;                           // FNV-1a of the library keys: the contexts of one sharded file must agree
+    bool shard_head_pending = false;                 // the next device chunk starts mid-file: k_shard_head runs on it first
+    bool shard_noguess = false;                      // ... and found no unique record start
+    const std::atomic<bool>* shard_abort = nullptr;  // another shard of the same call gave up: stop parsing
+    DevBuf shard_head;                               // the head bytes k_shard_head saved (<= carry_bytes)
+    int last_shards = 1, last_shard_fallback = 0;    // f2q_get_info "shards" / "shard_fallback"
     // state
     bool in_sample = false, closed = false;
     int sample_failed = F2Q_OK;        // a submit of this sample failed: every later submit / end of the sample reports it again
@@ -582,10 +590,26 @@ int ec_after_chunk(f2q_ctx* c) {
 
 // enqueue everything for one chunk that already sits in device memory at dptr[0, n)
 int process_device_chunk(f2q_ctx* c, const uint8_t* dptr, uint64_t n, int is_last) {
+    int rc;
+    if (c->shard_abort && c->shard_abort->load()) return fail(c, F2Q_EINVAL, "another shard of this file found no record start");
+    if (c->shard_head_pending && n) {
+        // first chunk of a shard that starts mid-file: guess its first record start (one round trip per shard), keep the
+        // head for the stitch and parse from the guess with line phase 0
+        c->shard_head_pending = false;
+        if ((rc = dev_alloc(c, c->shard_head, c->carry_cap + 256))) return rc;
+        k_shard_head<<<1, PREP_THREADS, 0, c->stream>>>(c->dS, dptr, n, reinterpret_cast<uint8_t*>(c->shard_head.p), c->carry_cap);
+        c->launches++;
+        CU(c, cudaGetLastError());
+        unsigned long long h = 0; uint32_t ok = 0;
+        CU(c, cudaMemcpyAsync(&h, &c->dS->head_len, 8, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaMemcpyAsync(&ok, &c->dS->head_ok, 4, cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaStreamSynchronize(c->stream));
+        if (!ok) { c->shard_noguess = true; return fail(c, F2Q_EINVAL, "no unique record start at the head of a shard"); }
+        dptr += h; n -= h;                                              // (n > h: the guess needs two whole records behind it)
+    }
     const uint64_t addr = reinterpret_cast<uint64_t>(dptr);
     const uint64_t delta = n ? (addr & 127ull) : 0;
     const uint8_t* base = n ? reinterpret_cast<const uint8_t*>(addr - delta) : reinterpret_cast<const uint8_t*>(c->carry.p);
-    int rc;
     if (!c->ch_decided) {
         // device chunks: sniff the record length (4 KiB of the first chunk) to size the tile rows — ONCE per context, so that
         // back-to-back samples have no host round trip (the geometry only affects speed, never results)
@@ -870,7 +894,7 @@ F2Q_EXPORT void f2q_destroy(f2q_ctx* c) {
     for (auto& b : c->lib_bufs) b.release();
     c->result.release(); c->carry.release(); c->status.release(); c->status_stitch.release(); c->queue.release(); c->gqueue.release();
     c->seg_count.release(); c->spec_rec.release(); c->spec_scratch.release(); c->slow_args.release(); c->synth_guides.release();
-    c->ec_slots.release(); c->ec_counts.release(); c->ec_arena.release(); c->ec_meta.release(); c->ec_pk.release(); c->ec_compact.release(); c->memo.release();
+    c->ec_slots.release(); c->ec_counts.release(); c->ec_arena.release(); c->ec_meta.release(); c->ec_pk.release(); c->ec_compact.release(); c->memo.release(); c->shard_head.release();
     for (auto& p : c->ec_pend) if (p.ev) cudaEventDestroy(p.ev);
     for (auto e : c->ec_events) cudaEventDestroy(e);
     if (c->ec_meta_host) cudaFreeHost(c->ec_meta_host);
@@ -1292,6 +1316,14 @@ F2Q_EXPORT int f2q_set_library(f2q_ctx* c, const uint8_t* key_bytes, const uint6
     c->T.slot_mask = cap - 1; c->T.n_fast = (uint32_t)fk.size(); c->T.n_keys = n_keys; c->T.ghash_mask = gcap - 1;
     c->T.n_generic = n_generic; c->T.generic_len_mask = gmask;
     c->n_keys = n_keys;
+    {
+        // FNV-1a over every key length and key byte, in library order
+        uint64_t lh = 1469598103934665603ull;
+        auto mix = [&](uint64_t v, int nb) { for (int b = 0; b < nb; b++) lh = (lh ^ ((v >> (8 * b)) & 0xFF)) * 1099511628211ull; };
+        mix(n_keys, 4);
+        for (uint32_t i = 0; i < n_keys; i++) { mix(off[i + 1] - off[i], 8); for (uint64_t k = off[i]; k < off[i + 1]; k++) mix(bytes[k], 1); }
+        c->lib_hash = lh;
+    }
     c->result.release();
     if ((rc = dev_alloc(c, c->result, ((size_t)n_keys + 5) * 8))) return rc;
     c->spec_scratch.release();
@@ -1325,6 +1357,8 @@ F2Q_EXPORT int f2q_begin_sample(f2q_ctx* c) {
         c->ec_drained = false; c->ec_merged = false;
     }
     c->in_sample = true; c->closed = false; c->sample_failed = F2Q_OK;
+    c->last_shards = 1; c->last_shard_fallback = 0;
+    c->shard_head_pending = false; c->shard_noguess = false;
     return F2Q_OK;
 }
 
@@ -1357,7 +1391,8 @@ F2Q_EXPORT int f2q_submit_device(f2q_ctx* c, const void* dptr, uint64_t nbytes, 
 static int submit_host(f2q_ctx* c, const uint8_t* host_chunk, uint64_t nbytes, int is_last, cudaEvent_t host_done) {
     int rc;
     if ((rc = ensure_staging(c))) return rc;
-    if (!c->ch_decided && nbytes) { decide_ch(c, host_chunk, (size_t)std::min<uint64_t>(nbytes, 4096)); c->ch_from_device = false; }
+    // (a shard that starts mid-file sniffs on the device, behind its head)
+    if (!c->ch_decided && nbytes && !c->shard_head_pending) { decide_ch(c, host_chunk, (size_t)std::min<uint64_t>(nbytes, 4096)); c->ch_from_device = false; }
     uint64_t done = 0;
     do {
         const uint64_t len = std::min<uint64_t>(c->stage_bytes, nbytes - done);
@@ -1441,6 +1476,23 @@ size_t pread_parallel(int fd, uint8_t* buf, size_t want, uint64_t off, int T) {
     return n;
 }
 
+// the page-locked ring lives with the context (allocated on first use), with the staging slots behind it
+int ensure_ring(f2q_ctx* c) {
+    int rc;
+    if (!c->file_ring) c->file_ring = new FileRing();
+    FileRing& R = *c->file_ring;
+    if (!R.buf[0]) {
+        R.bytes = 32u << 20;
+        for (int k = 0; k < FileRing::N; k++) {
+            void* p = nullptr;
+            if ((rc = f2q_host_alloc_near(&p, R.bytes + 65536, c->device, 0, nullptr))) return fail(c, rc, f2q_last_error(nullptr));
+            R.buf[k] = static_cast<uint8_t*>(p);
+            if (cudaEventCreateWithFlags(&R.done[k], cudaEventDisableTiming) != cudaSuccess) return fail(c, F2Q_ECUDA, "cudaEventCreate failed");
+        }
+    }
+    return ensure_staging(c);
+}
+
 const uint8_t* last_newline(const uint8_t* p, size_t n) { return static_cast<const uint8_t*>(memrchr(p, '\n', n)); }
 
 // BGZF block at p (>= 18 bytes available): total block size, or 0 when this is not a BGZF member header
@@ -1462,8 +1514,9 @@ const uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 0x08, 0x04, 0, 0, 0, 0, 0, 0xff, 0x06,
 // of k_inflate_bgzf_lanes per batch (<= 1 GiB compressed, <= 3 GiB of output, <= 65 536 blocks: tens of thousands of lanes) writes the FASTQ text straight
 // into the buffer process_device_chunk parses.  Two staging / output buffers: the next batch is read and copied while the
 // previous one is inflated and parsed.  Stops at the first thing that is not a whole BGZF block (a foreign gzip member, a
-// truncated block) and reports the file offset there: the host reader takes over from that offset.
-int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t* total, uint64_t* resume_off, bool* finished) {
+// truncated block) and reports the file offset there: the host reader takes over from that offset.  Reads the file bytes
+// [begin, end) only (a shard of f2q_submit_file_sharded: whole blocks); `finished` = that range was whole BGZF blocks.
+int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t begin, uint64_t end, uint64_t* total, uint64_t* resume_off, bool* finished) {
     int rc;
     const int T = std::max(1, std::min(threads, 8));
     static const bool debug = getenv("F2Q_DEBUG_INGEST") != nullptr;   // developer lap timers: where the host thread spends its time
@@ -1474,12 +1527,9 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t* tot
     // blocks, however few blocks it has), so a small last batch costs as much as a full one.  The staging buffers follow the
     // file: a 100 MB sample does not take the 8 GB a 10 GB one is given (many contexts may share the GPU)
     size_t comp_target = GZ_COMP_BYTES;
-    {
-        struct stat sb;
-        if (fstat(fd, &sb) == 0 && sb.st_size > 0) {
-            const size_t usable = GZ_COMP_BYTES - R.bytes - 65536, nbatch = ((size_t)sb.st_size + usable - 1) / usable;
-            comp_target = std::min(GZ_COMP_BYTES, ((size_t)sb.st_size + nbatch - 1) / nbatch + 2 * R.bytes + 65536);
-        }
+    if (end > begin) {
+        const size_t span = (size_t)(end - begin), usable = GZ_COMP_BYTES - R.bytes - 65536, nbatch = (span + usable - 1) / usable;
+        comp_target = std::min(GZ_COMP_BYTES, (span + nbatch - 1) / nbatch + 2 * R.bytes + 65536);
     }
     const size_t out_target = std::min(GZ_OUT_BYTES, std::max<size_t>(6 * comp_target, 8 * R.bytes));
     const double t_alloc0 = now();
@@ -1493,7 +1543,7 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t* tot
     }
     const size_t out_cap = c->gz_out[0].n - 65536 - 256;               // (what the buffers hold: at least the targets)
     const double t_alloc = now() - t_alloc0;
-    uint64_t off = 0;                                                  // file offset of the next unread byte
+    uint64_t off = begin;                                              // file offset of the next unread byte
     std::vector<uint8_t> carry;                                        // the head of a block whose rest is in the next piece
     bool eof = false, stop = false;
     int batch = 0;
@@ -1521,9 +1571,9 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t* tot
             carry.clear();
             if (have < R.bytes) {
                 t0 = now();
-                const size_t want = R.bytes - have, g = pread_parallel(fd, buf + have, want, off, T);
+                const size_t want = (size_t)std::min<uint64_t>(R.bytes - have, end - off), g = pread_parallel(fd, buf + have, want, off, T);
                 t_read += now() - t0;
-                if (g < want) eof = true;
+                if (g < want || off + g == end) eof = true;
                 have += g; off += g;
             }
             t0 = now();
@@ -1610,19 +1660,8 @@ F2Q_EXPORT int f2q_submit_file(f2q_ctx* c, const char* path, int is_gzip, uint64
     FILE* f = fopen(path, "rb");
     if (!f) return fail(c, F2Q_EINVAL, std::string("cannot open ") + path + ": " + strerror(errno));
     setvbuf(f, nullptr, _IONBF, 0);
-    // the ring lives with the context
-    if (!c->file_ring) c->file_ring = new FileRing();
+    if ((rc = ensure_ring(c))) { fclose(f); return rc; }
     FileRing& R = *c->file_ring;
-    if (!R.buf[0]) {
-        R.bytes = 32u << 20;
-        for (int k = 0; k < FileRing::N; k++) {
-            void* p = nullptr;
-            if ((rc = f2q_host_alloc_near(&p, R.bytes + 65536, c->device, 0, nullptr))) { fclose(f); return fail(c, rc, f2q_last_error(nullptr)); }
-            R.buf[k] = static_cast<uint8_t*>(p);
-            if (cudaEventCreateWithFlags(&R.done[k], cudaEventDisableTiming) != cudaSuccess) { fclose(f); return fail(c, F2Q_ECUDA, "cudaEventCreate failed"); }
-        }
-    }
-    if ((rc = ensure_staging(c))) { fclose(f); return rc; }
     uint64_t total = 0, lines_left = limit_lines;
     bool stop = false;                                                 // preprocess mode: the line limit was reached
     // cut `n` bytes at the line limit; returns the bytes to submit
@@ -1690,7 +1729,7 @@ F2Q_EXPORT int f2q_submit_file(f2q_ctx* c, const char* path, int is_gzip, uint64
         struct stat sb;
         if (fstat(fileno(f), &sb) == 0 && sb.st_size >= 28 && pread(fileno(f), tailb, 28, sb.st_size - 28) == 28 && memcmp(tailb, BGZF_EOF, 28) == 0) {
             uint64_t resume = 0; bool finished = false;
-            if ((rc = submit_bgzf_gpu(c, f, R, threads, &total, &resume, &finished))) { fclose(f); return rc; }
+            if ((rc = submit_bgzf_gpu(c, f, R, threads, 0, (uint64_t)sb.st_size, &total, &resume, &finished))) { fclose(f); return rc; }
             if (finished) {
                 fclose(f);
                 rc = ring_get(c, R, &buf, &idx);
@@ -2289,6 +2328,270 @@ F2Q_EXPORT int f2q_ec_merge(f2q_ctx** ctxs, int n) {
     return F2Q_OK;
 }
 
+// ---- one file, several contexts ------------------------------------------------------------------------------------
+// f2q_submit_file_sharded (DESIGN.md §5): the file is cut into byte ranges, one per context, and every context parses its
+// range on its own host thread and its own stream, exactly as f2q_submit_file would.  A range that starts mid-file guesses
+// its first record start on the device (k_shard_head); the guesses are verified on the host once every range is parsed,
+// the bytes around the cuts (the head before each guess, the partial record behind each range's last whole record) are
+// parsed on ctxs[0] in file order, and the other contexts' results are added into ctxs[0].  Anything that cannot be split
+// or verified is parsed again, whole, on ctxs[0].
+namespace {
+
+constexpr uint64_t SHARD_MIN_BYTES = 64ull << 20;
+
+// file offsets of the blocks of a bgzip file, from their 18-byte headers alone; false unless the file is whole BGZF blocks
+// that end with the end-of-file block (a foreign gzip member or a truncated block leave nothing to cut at)
+bool bgzf_block_starts(int fd, uint64_t size, std::vector<uint64_t>& starts) {
+    starts.clear();
+    uint8_t hdr[18];
+    for (uint64_t off = 0; off < size;) {
+        if (size - off < 28 || pread(fd, hdr, 18, (off_t)off) != 18) return false;
+        const size_t bs = bgzf_block_size(hdr, 18);
+        if (!bs || bs > size - off) return false;
+        starts.push_back(off);
+        off += bs;
+    }
+    uint8_t eof[28];
+    return !starts.empty() && starts.back() == size - 28 && pread(fd, eof, 28, (off_t)(size - 28)) == 28 && memcmp(eof, BGZF_EOF, 28) == 0;
+}
+
+struct ShardJob { uint64_t beg = 0, end = 0; bool first = false, last = false; int threads = 1; int rc = F2Q_OK; uint64_t bytes = 0; };
+
+// one range of the file -> this context's sample: the first range is parsed as the start of the stream, the last one closes
+// it, the others end with their partial record carried (k_carry) and begin with k_shard_head
+int shard_run(f2q_ctx* c, const char* path, bool gz, ShardJob& J) {
+    int rc = check_ctx(c); if (rc) return rc;
+    FILE* f = fopen(path, "rb");
+    if (!f) return fail(c, F2Q_EINVAL, std::string("cannot open ") + path + ": " + strerror(errno));
+    setvbuf(f, nullptr, _IONBF, 0);
+    if ((rc = ensure_ring(c))) { fclose(f); return rc; }
+    FileRing& R = *c->file_ring;
+    c->shard_head_pending = !J.first;
+    if (!gz) {
+        // plain file: pread straight into this context's ring
+        const int fd = fileno(f);
+        for (uint64_t off = J.beg; off < J.end && !rc;) {
+            uint8_t* buf; int idx;
+            if ((rc = ring_get(c, R, &buf, &idx))) break;
+            const size_t want = (size_t)std::min<uint64_t>(R.bytes, J.end - off), got = pread_parallel(fd, buf, want, off, J.threads);
+            if (got < want) { rc = fail(c, F2Q_EINVAL, std::string(path) + ": the file ended early (did it change?)"); break; }
+            off += got; J.bytes += got;
+            rc = ring_submit(c, R, idx, got, (J.last && off == J.end) ? 1 : 0);
+        }
+    } else {
+        uint64_t resume = 0; bool finished = false;
+        rc = submit_bgzf_gpu(c, f, R, J.threads, J.beg, J.end, &J.bytes, &resume, &finished);
+        if (!rc && !finished) { c->shard_noguess = true; rc = fail(c, F2Q_EINVAL, "a shard is not whole BGZF blocks"); }
+        if (!rc && J.last) rc = process_device_chunk(c, nullptr, 0, 1);
+    }
+    fclose(f);
+    c->shard_head_pending = false;
+    return rc;
+}
+
+int copy_to(f2q_ctx* dst, void* d, const f2q_ctx* src, const void* s, size_t n) {
+    if (!n) return F2Q_OK;
+    if (dst->device == src->device) CU(dst, cudaMemcpyAsync(d, s, n, cudaMemcpyDeviceToDevice, dst->stream));
+    else CU(dst, cudaMemcpyPeerAsync(d, dst->device, s, src->device, n, dst->stream));
+    return F2Q_OK;
+}
+
+// the arena keys of one context's Extract+Count table, added into `extra` (host)
+int ec_arena_collect(f2q_ctx* c, std::map<std::string, uint64_t>& extra) {
+    std::vector<unsigned long long> ap; std::vector<uint8_t> ar;
+    int rc = ec_arena_fetch(c, ap, ar); if (rc) return rc;
+    for (size_t k = 0; k + 1 < ap.size(); k += 2) {
+        const uint64_t off = (ap[k] - 1) >> 24, len = (ap[k] - 1) & 0xFFFFFF;
+        extra[std::string(reinterpret_cast<const char*>(ar.data() + off), len)] += ap[k + 1];
+    }
+    return F2Q_OK;
+}
+
+}  // namespace
+
+F2Q_EXPORT int f2q_submit_file_sharded(f2q_ctx** ctxs, int n, const char* path, int is_gzip, const uint64_t* cuts, int threads,
+                                       int* complete, uint64_t* bytes_out) {
+    if (!ctxs || n < 1 || !ctxs[0]) return fail(nullptr, F2Q_EINVAL, "f2q_submit_file_sharded: no contexts");
+    f2q_ctx* c0 = ctxs[0];
+    int rc;
+    for (int i = 0; i < n; i++) {
+        f2q_ctx* c = ctxs[i];
+        if (!c) return fail(c0, F2Q_EINVAL, "null context");
+        for (int j = 0; j < i; j++) if (ctxs[j] == c) return fail(c0, F2Q_EINVAL, "a context appears twice");
+        if ((rc = check_ctx(c))) return rc;
+        if (!c->in_sample) return fail(c0, F2Q_ESTATE, "f2q_submit_file_sharded: context " + std::to_string(i) + " is not inside a sample");
+        if (c->sample_failed) return c->sample_failed;
+        if (c->closed) return fail(c0, F2Q_ESTATE, "f2q_submit_file_sharded: the stream of context " + std::to_string(i) + " is already closed");
+        if (memcmp(&c->cfg, &c0->cfg, sizeof(f2q_config)) != 0 || c->n_keys != c0->n_keys || c->lib_hash != c0->lib_hash)
+            return fail(c0, F2Q_EINVAL, "f2q_submit_file_sharded: context " + std::to_string(i) + " has another configuration or library than context 0");
+    }
+    if (!path) return fail(c0, F2Q_EINVAL, "null path");
+    if (cuts) for (int k = 1; k + 1 < n; k++) if (cuts[k] < cuts[k - 1]) return fail(c0, F2Q_EINVAL, "cuts must not decrease");
+    if (complete) *complete = 1;
+    if (bytes_out) *bytes_out = 0;
+    const bool gz = is_gzip != 0;
+    // ---- the plan: range bounds [0 = b_0 < b_1 < ... < b_s = size], empty ranges dropped
+    std::vector<uint64_t> bounds(1, 0);
+    bool shardable = true;
+    {
+        FILE* f = fopen(path, "rb");
+        if (!f) return fail(c0, F2Q_EINVAL, std::string("cannot open ") + path + ": " + strerror(errno));
+        struct stat sb;
+        const uint64_t size = fstat(fileno(f), &sb) == 0 ? (uint64_t)sb.st_size : 0;
+        std::vector<uint64_t> starts;
+        if (gz) {
+            // only bgzip can be cut (at block starts; ordinary gzip is one deflate stream), and only when inflated on the device
+            uint8_t h[18];
+            shardable = c0->gpu_inflate && pread(fileno(f), h, 18, 0) == 18 && bgzf_block_size(h, 18) && bgzf_block_starts(fileno(f), size, starts);
+        }
+        fclose(f);
+        const int want = cuts ? n : (int)std::min<uint64_t>((uint64_t)n, std::max<uint64_t>(1, size / SHARD_MIN_BYTES));
+        for (int k = 1; shardable && k < want; k++) {
+            uint64_t x = std::min(size, cuts ? cuts[k - 1] : size / want * k);
+            if (gz) {
+                // the next block start; none before the end-of-file block: the end of the file
+                auto it = std::lower_bound(starts.begin(), starts.end() - 1, x);
+                x = it == starts.end() - 1 ? size : *it;
+            }
+            if (x > bounds.back() && x < size) bounds.push_back(x);
+        }
+        bounds.push_back(size);
+    }
+    const int ns = (int)bounds.size() - 1;
+    // ---- the other contexts end empty and closed; ctxs[0] takes the whole file when there is one range or a fallback
+    auto close_others = [&]() -> int {
+        for (int k = 1; k < n; k++) {
+            f2q_ctx* c = ctxs[k];
+            c->ch_from_device = false;                                  // (its geometry was sniffed behind a shard head)
+            int r = f2q_begin_sample(c); if (r) return r;
+            c->closed = true;
+        }
+        return F2Q_OK;
+    };
+    auto whole_on_ctx0 = [&](bool fallback) -> int {
+        int r = close_others(); if (r) return r;
+        if (fallback && (r = f2q_begin_sample(c0))) return r;
+        r = f2q_submit_file(c0, path, is_gzip, 0, threads, complete, bytes_out);
+        c0->last_shards = 1; c0->last_shard_fallback = fallback ? 1 : 0;
+        return r;
+    };
+    if (!shardable || ns < 2) return whole_on_ctx0(!shardable);
+
+    // ---- every range on its own context and host thread
+    std::atomic<bool> abort{false};
+    std::vector<ShardJob> J(ns);
+    for (int k = 0; k < ns; k++) {
+        J[k].beg = bounds[k]; J[k].end = bounds[k + 1]; J[k].first = k == 0; J[k].last = k == ns - 1;
+        J[k].threads = std::max(1, threads / ns);
+        ctxs[k]->shard_abort = &abort; ctxs[k]->shard_noguess = false;
+    }
+    auto run = [&](int k) {
+        J[k].rc = shard_run(ctxs[k], path, gz, J[k]);
+        if (ctxs[k]->shard_noguess) abort = true;                       // the others need not finish: the file is parsed again
+    };
+    {
+        std::vector<std::thread> pool;
+        for (int k = 1; k < ns; k++) pool.emplace_back(run, k);
+        run(0);
+        for (auto& t : pool) t.join();
+    }
+    bool noguess = false;
+    for (int k = 0; k < ns; k++) { ctxs[k]->shard_abort = nullptr; noguess = noguess || ctxs[k]->shard_noguess; }
+    if (noguess) return whole_on_ctx0(true);
+    for (int k = 0; k < ns; k++)
+        if (J[k].rc) { if (k) c0->err = ctxs[k]->err; return J[k].rc; }
+    std::vector<DevState> S(ns);
+    bool dev_error = false;                                            // a range failed on the device (a record longer than carry_bytes ...)
+    for (int k = 0; k < ns; k++) {
+        f2q_ctx* c = ctxs[k];
+        uint32_t err = 0;
+        cudaSetDevice(c->device);
+        CU(c, cudaStreamSynchronize(c->stream));
+        CU(c, cudaMemcpy(&S[k], c->dS, sizeof(DevState), cudaMemcpyDeviceToHost));
+        CU(c, cudaMemcpy(&err, c->d_error, 4, cudaMemcpyDeviceToHost));
+        dev_error = dev_error || err || S[k].error;
+    }
+    // ---- verification.  Records are every 4 lines from byte 0.  Range 0 starts at byte 0, so at line phase 0.  When range k-1
+    // is parsed at the right phase, its carried partial record holds tail_nl[k-1] lines of the record that range k's head
+    // completes; range k's guess is a record start exactly when the head adds the missing lines, (tail_nl[k-1] + head_nl[k])
+    // % 4 == 0 (head_nl is 1..4, so the head is exactly those lines).  Then range k is parsed at the right phase too: by
+    // induction every guess is right, and every record is parsed exactly once, either inside a range or from a tail + head.
+    // A range that failed on the device fails the sample: no check, no stitch, its error words reach ctxs[0] with the sum below
+    // (a second pass on ctxs[0] could hide the failure where its own chunks happen to be cut elsewhere).
+    for (int k = 1; k < ns && !dev_error; k++)
+        if (!S[k].head_ok || (S[k - 1].tail_nl + S[k].head_nl) % 4 != 0) return whole_on_ctx0(true);
+
+    // ---- stitch: ctxs[0] (carrying range 0's tail) is fed H1, T1, H2, ..., T(s-2), H(s-1) and closed
+    std::vector<std::vector<uint8_t>> piece;
+    for (int k = 1; k < ns && !dev_error; k++) {
+        f2q_ctx* c = ctxs[k];
+        cudaSetDevice(c->device);
+        piece.emplace_back(S[k].head_len);
+        if (S[k].head_len) CU(c0, cudaMemcpy(piece.back().data(), c->shard_head.p, S[k].head_len, cudaMemcpyDeviceToHost));
+        if (k == ns - 1) break;
+        piece.emplace_back(S[k].tail_len);
+        if (S[k].tail_len) CU(c0, cudaMemcpy(piece.back().data(), c->carry.p, S[k].tail_len, cudaMemcpyDeviceToHost));
+    }
+    if ((rc = check_ctx(c0))) return rc;
+    for (auto& p : piece)
+        if (!p.empty() && (rc = submit_host(c0, p.data(), p.size(), 0, nullptr))) { c0->sample_failed = rc; return rc; }
+    if ((rc = process_device_chunk(c0, nullptr, 0, 1))) { c0->sample_failed = rc; return rc; }
+
+    // ---- sum: [counts | stats] and the error words of every other range into ctxs[0] (their streams are idle: synchronised above)
+    const uint64_t nw = (uint64_t)c0->n_keys + 5;
+    DevBuf recv, recv_pk;
+    auto release = [&]() { cudaSetDevice(c0->device); cudaStreamSynchronize(c0->stream); recv.release(); recv_pk.release(); };
+    if ((rc = dev_alloc(c0, recv, nw * 8 + 16))) return rc;
+    uint32_t* recv_err = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(recv.p) + nw * 8);
+    for (int k = 1; k < ns; k++) {
+        f2q_ctx* c = ctxs[k];
+        if ((rc = copy_to(c0, recv.p, c, c->result.p, nw * 8)) || (rc = copy_to(c0, recv_err, c, c->d_error, 4)) ||
+            (rc = copy_to(c0, recv_err + 1, c, &c->dS->error, 4))) { release(); return rc; }
+        k_shard_sum<<<(unsigned)std::min<uint64_t>((nw + 255) / 256, (uint64_t)c0->sm_count * 4), 256, 0, c0->stream>>>(
+            reinterpret_cast<unsigned long long*>(c0->result.p), reinterpret_cast<const unsigned long long*>(recv.p), nw, c0->d_error, c0->dS, recv_err);
+        c0->launches++;
+        CU(c0, cudaGetLastError());
+    }
+    if (c0->cfg.mode == F2Q_MODE_EXTRACT_COUNT) {
+        // Extract+Count: every other packed table compacted on its device, copied over and inserted into ctxs[0]'s (counts
+        // add); the few byte-arena keys of every context, ctxs[0]'s own included, merge on the host (as f2q_ec_merge does)
+        std::map<std::string, uint64_t> extra;
+        CU(c0, cudaStreamSynchronize(c0->stream));
+        if ((rc = ec_arena_collect(c0, extra))) { release(); return rc; }
+        for (int k = 1; k < ns; k++) {
+            f2q_ctx* c = ctxs[k];
+            uint64_t npk = 0;
+            cudaSetDevice(c->device);
+            if ((rc = ec_arena_collect(c, extra)) || (rc = ec_compact_packed(c, &npk))) { c0->err = c->err; release(); return rc; }
+            cudaSetDevice(c0->device);
+            if (!npk) continue;
+            if ((rc = dev_alloc(c0, recv_pk, npk * 16)) || (rc = copy_to(c0, recv_pk.p, c, reinterpret_cast<const uint8_t*>(c->ec_compact.p) + 16, npk * 16)) ||
+                (rc = ec_reserve(c0, npk, 0, 0))) { release(); return rc; }
+            k_ec_merge_pairs<<<(unsigned)std::min<uint64_t>((npk + 255) / 256, (uint64_t)c0->sm_count * 16), 256, 0, c0->stream>>>(
+                c0->E, outputs_of(c0), reinterpret_cast<const unsigned long long*>(recv_pk.p), npk);
+            c0->launches++;
+            CU(c0, cudaGetLastError());
+            if ((rc = ec_after_chunk(c0))) { release(); return rc; }
+            CU(c0, cudaStreamSynchronize(c0->stream));                 // (recv_pk is refilled for the next context)
+        }
+        c0->ec_extra_keys.clear(); c0->ec_extra_off.assign(1, 0); c0->ec_extra_cnt.clear();
+        for (auto& kv : extra) {
+            c0->ec_extra_keys.insert(c0->ec_extra_keys.end(), kv.first.begin(), kv.first.end());
+            c0->ec_extra_off.push_back(c0->ec_extra_keys.size());
+            c0->ec_extra_cnt.push_back(kv.second);
+        }
+        c0->ec_merged = true; c0->ec_drained = false;
+    }
+    release();
+    if ((rc = close_others())) return rc;
+    if ((rc = check_ctx(c0))) return rc;
+    c0->last_shards = ns; c0->last_shard_fallback = 0;
+    uint64_t total = 0;
+    for (auto& j : J) total += j.bytes;
+    if (bytes_out) *bytes_out = total;
+    return F2Q_OK;
+}
+
 // ---- memory helpers --------------------------------------------------------------------------------------
 F2Q_EXPORT int f2q_host_alloc(void** ptr, uint64_t nbytes) {
     if (!ptr) return F2Q_EINVAL;
@@ -2416,6 +2719,8 @@ F2Q_EXPORT int f2q_get_info(f2q_ctx* c, const char* name, int64_t* value) {
     else if (n == "hist") *value = c->hist_used;
     else if (n == "seed_parts") *value = c->T.seed_ncombo ? (int64_t)c->T.seed_parts : 0;
     else if (n == "flex_table") *value = c->T.fx_slots ? 1 : 0;
+    else if (n == "shards") *value = c->last_shards;
+    else if (n == "shard_fallback") *value = c->last_shard_fallback;
     else if (n == "generic_reads") {
         if (c->in_sample) return fail(c, F2Q_ESTATE, "generic_reads is known once the sample has finished");
         unsigned long long v = 0;

@@ -138,6 +138,8 @@ struct DevState {
     uint32_t spec_commits, spec_fallbacks;   // chunks of this sample whose speculation held / that the exact kernel parsed
     unsigned long long memo_lookups, memo_hits;
     unsigned long long generic_reads;   // reads the generic read queue took this sample (k_generic_queue, f2q_get_info)
+    unsigned long long head_len;   // k_shard_head: bytes before the guessed first record of a shard (its head)
+    uint32_t head_nl, head_ok;     // ... newlines in the head (1-4); 1 when exactly one candidate start was accepted
     unsigned long long dbg[8];     // diagnostics (F2Q_DEBUG=1): failed mbarrier tries per wait site, look-back rounds / spins
 };
 

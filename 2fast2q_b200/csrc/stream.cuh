@@ -111,6 +111,71 @@ __global__ void __launch_bounds__(PREP_THREADS) k_carry(DevState* S, const uint8
 }
 
 // ------------------------------------------------------------------------------------------------
+// One file on several contexts (f2q_submit_file_sharded): every shard but the first starts at an arbitrary byte offset.
+// k_shard_head guesses where its first record starts, from the local record shape alone: the candidates are the bytes
+// behind the 1st..4th newline of the shard, and a candidate is accepted when the two records starting there look like
+// FASTQ records ('@' header, '+' third line, sequence and quality lines of equal length, the next record starting with '@').
+// Exactly one accepted candidate is the guess h; the head [0, h) (1-4 newlines) is saved for the stitch and the shard is
+// parsed from h with line phase 0.  The guess is only a guess: the host verifies it against the shard before (DESIGN.md §5).
+// ------------------------------------------------------------------------------------------------
+constexpr int SHARD_HEAD_NL = 12;              // newlines candidate 4 needs: 4 to reach it + 8 for its two records
+
+__global__ void __launch_bounds__(PREP_THREADS) k_shard_head(DevState* S, const uint8_t* __restrict__ buf, uint64_t n,
+                                                             uint8_t* __restrict__ head, uint64_t head_cap) {
+    __shared__ uint64_t nlpos[SHARD_HEAD_NL];
+    __shared__ uint64_t s_h;
+    const uint32_t tid = threadIdx.x;
+    if (tid < 32) {
+        // the first SHARD_HEAD_NL newlines, one warp, 32 x 16 bytes per step (as k_prepare)
+        uint32_t seen = 0;
+        for (uint64_t pos = 0; pos < n && seen < (uint32_t)SHARD_HEAD_NL; pos += 512) {
+            const uint64_t a = pos + (uint64_t)tid * 16;
+            uint32_t mask = 0;
+            for (int b = 0; b < 16; b++) if (a + b < n && buf[a + b] == '\n') mask |= 1u << b;
+            const uint32_t c = __popc(mask);
+            uint32_t incl = c;
+            for (int d = 1; d < 32; d <<= 1) { uint32_t y = __shfl_up_sync(0xffffffffu, incl, d); if (tid >= (uint32_t)d) incl += y; }
+            uint32_t r = seen + incl - c;
+            for (uint32_t m = mask; m && r < (uint32_t)SHARD_HEAD_NL; m &= m - 1) nlpos[r++] = a + (uint64_t)(__ffs(m) - 1);
+            seen += __shfl_sync(0xffffffffu, incl, 31);
+        }
+        __syncwarp();
+        if (tid == 0) {
+            uint32_t accepted = 0, nl = 0; uint64_t h = 0;
+            if (seen >= (uint32_t)SHARD_HEAD_NL) {
+                for (uint32_t i = 1; i <= 4; i++) {
+                    const uint64_t* L = nlpos + i - 1;          // L[0] ends the line before the candidate, L[1..8] its 8 lines
+                    bool ok = true;
+                    for (int r = 0; r < 2 && ok; r++) {
+                        const uint64_t* q = L + 4 * r;
+                        ok = buf[q[0] + 1] == '@' && buf[q[2] + 1] == '+' && q[2] - q[1] == q[4] - q[3];
+                    }
+                    ok = ok && L[8] + 1 < n && buf[L[8] + 1] == '@';
+                    if (ok) { accepted++; nl = i; h = L[0] + 1; }
+                }
+            }
+            const bool good = accepted == 1 && h <= head_cap;
+            S->head_ok = good ? 1u : 0u; S->head_nl = good ? nl : 0u; S->head_len = good ? h : 0ull;
+            s_h = good ? h : 0ull;
+        }
+    }
+    __syncthreads();
+    const uint64_t h = s_h;
+    for (uint64_t i = tid; i < h; i += PREP_THREADS) head[i] = buf[i];
+}
+
+// the result of another shard's context (copied next to this one: peer copy or same-device copy) is added to this context's
+// result vector; its error words are ORed into this context's, so that a failure in any shard fails the whole sample
+__global__ void __launch_bounds__(256) k_shard_sum(unsigned long long* __restrict__ result, const unsigned long long* __restrict__ other, uint64_t n_words,
+                                                   uint32_t* error, DevState* S, const uint32_t* __restrict__ other_errors) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_words; i += (uint64_t)gridDim.x * blockDim.x) result[i] += other[i];
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        if (other_errors[0]) atomicOr(error, other_errors[0]);
+        if (other_errors[1]) atomicOr(&S->error, other_errors[1]);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // GPU inflate of bgzip (BGZF) input: one thread per block (inflate_core.h).  The blocks of a chunk are independent, their
 // compressed sizes come from the headers and their output offsets from the trailers, so thousands decode at once straight
 // into the buffer the streaming kernel parses; only the COMPRESSED bytes cross PCIe.

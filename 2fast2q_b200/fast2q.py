@@ -389,18 +389,19 @@ def _config_of(param):
         sys.exit()
 
 
-def _engine_for(param, features, device):
-    """cached per thread: creating a context and uploading a 100k-guide library once per file would dominate small files"""
+def _engine_for(param, features, device, slot=0):
+    """cached per thread: creating a context and uploading a 100k-guide library once per file would dominate small files.
+    `slot` keeps several engines of one thread apart (split_file_native: one per shard, several may share a device)"""
     cfg = _config_of(param)
     keys = list(features.keys()) if param["Running Mode"] == "C" else None
-    sig = (device, bytes(cfg), None if keys is None else hash(tuple(keys)))
+    sig = (device, bytes(cfg), None if keys is None else hash(tuple(keys)), slot)
     cache = getattr(_tls, "engines", None)
     if cache is None:
         cache = _tls.engines = {}
     if sig not in cache:
-        for old in cache.values():
+        for old_sig in [k for k in cache if k[-1] == slot]:
+            old = cache.pop(old_sig)
             old[0].close(); old[1].free()
-        cache.clear()
         # the device memo of resolved non-exact keys (the reference's passed_reads / failed_reads): real screens repeat them
         eng = _lib.Engine(cfg, device, memo_entries=1 << 20) if keys is not None else _lib.Engine(cfg, device)
         if keys is not None:
@@ -895,6 +896,48 @@ def split_file_counter(raw, features, param, n_gpus):
     return merged, stats, complete
 
 
+def split_file_native(raw, features, param, devices):
+    """File-Split mode on several GPUs: one plain or bgzip file as ONE sample, parsed by one cached engine per entry of
+    `devices` (entries may repeat a device).  Each engine reads and parses its own byte range of the file natively
+    (f2q_submit_file_sharded); the first one ends with the whole sample.  Writes <sample>_reads.csv as aligner does."""
+    tempo = time.perf_counter()
+    _derive_positions(param)
+    engines = [_engine_for(param, features, int(d), slot=k)[0] for k, d in enumerate(devices)]
+    gz = os.path.splitext(raw)[1] == ".gz"
+
+    def end_all():
+        for e in engines:
+            try:
+                e.end()
+            except _lib.F2QError:
+                pass
+
+    for e in engines:
+        e.begin()
+    try:
+        complete, _ = _lib.submit_file_sharded(engines, raw, gz, threads=_INFLATE_WORKERS)
+    except _lib.F2QError as e:
+        end_all()
+        if e.code == -1 and "corrupted gzip" in str(e):
+            colourful_errors("WARNING", f"{raw} is an incomplete or corrupted gzip file. ({e})")
+            return
+        if e.code == -1 and "cannot open" in str(e):
+            raise OSError(str(e)) from None
+        raise
+    except BaseException:
+        end_all()
+        raise
+    counts, local_read_stats = engines[0].end()
+    for e in engines[1:]:
+        e.end()                                              # (closed and empty: leaves the cached engine reusable)
+    if not complete:
+        colourful_errors("WARNING", f"{raw} is an incomplete or corrupted gzip file. Only partial processing might have occurred.")
+    if param["Running Mode"] == "C":
+        _write_sample_counts(raw, features, counts, local_read_stats, param, time.perf_counter() - tempo)
+    else:
+        write_sample(raw, _features_from(param, features, counts, engines[0]), local_read_stats, param, time.perf_counter() - tempo)
+
+
 def aligner_mp_dispenser(features, param, start=0):
     """processes every sample (fast2q.py:1619-1655).  File mode: `cpu` feeder threads take files from a queue, thread k
     drives GPU k mod n_gpus through its own context (samples are independent: no collective).  File-Split mode
@@ -910,10 +953,14 @@ def aligner_mp_dispenser(features, param, start=0):
             tempo = time.perf_counter()
             if SPLIT_NATIVE_SINGLE_GPU:
                 # The native ingest (parallel reads / BGZF-parallel inflate into pinned memory) feeds ONE context faster than
-                # the Python reader below can cut shards for eight (measured: 2.4 GB/s against 0.26 GB/s on a 5.9 GB file);
-                # one GPU parses far faster than any host reader delivers, so the file goes to one GPU.  Counts are the same
+                # the Python reader below can cut shards for eight (measured: 2.4 GB/s against 0.26 GB/s on a 5.9 GB file).
+                # With several GPUs a plain or bgzip file is cut natively instead: every GPU reads and parses its own byte
+                # range (split_file_native).  Ordinary gzip is one deflate stream with nowhere to cut: one GPU.  Counts are the same
                 try:
-                    aligner(0, raw, features, dict(param, device=0), reads_stats)
+                    if n_gpus > 1 and _input_kind([raw]) != "gzip":
+                        split_file_native(raw, features, dict(param, device=0), list(range(n_gpus)))
+                    else:
+                        aligner(0, raw, features, dict(param, device=0), reads_stats)
                 finally:
                     release_engines()
                 continue

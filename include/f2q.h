@@ -172,6 +172,28 @@ int f2q_submit(f2q_ctx* ctx, const uint8_t* host_chunk, uint64_t nbytes, int is_
  */
 int f2q_submit_file(f2q_ctx* ctx, const char* path, int is_gzip, uint64_t limit_lines, int threads, int* complete, uint64_t* bytes_out);
 
+/*
+ * One plain or bgzip file as ONE sample parsed by n contexts (on one device or several; no NCCL): the file is cut into byte
+ * ranges, context k parses range k on a host thread of its own (`threads` readers are divided among them), and on return
+ * ctxs[0] holds the whole sample — counts, statistics, the device error word and, in Extract+Count mode, the merged key
+ * table — so f2q_end_sample / f2q_end_sample_async / f2q_ec_size / f2q_ec_drain on ctxs[0] work as after f2q_submit_file.
+ * Every other context's sample is closed and empty.  *complete and *bytes_out mean what they mean for f2q_submit_file.
+ * Preconditions: n >= 1, no context twice (else F2Q_EINVAL); every context inside a freshly begun sample (else F2Q_ESTATE);
+ * all with the same f2q_config bytes and the same library (else F2Q_EINVAL).
+ * cuts: NULL splits the file evenly into ranges of at least 64 MiB (a small file uses fewer contexts), or n-1 non-decreasing
+ * file offsets (bgzip: rounded up to the next block start); empty ranges are dropped.
+ * Protocol: a range that starts mid-file guesses its first record start on the device (the one byte behind its 1st..4th
+ * newline where two records of FASTQ shape start); the bytes before it (its head) and the partial record behind the last
+ * whole record of the range before (its tail) are parsed on ctxs[0] in file order.  A guess is right exactly when the
+ * tail's newlines plus the head's are a multiple of 4; this is checked for every range, so by induction every record is
+ * parsed once at its true line phase.  The whole file is parsed again on ctxs[0] alone (the other samples restart empty)
+ * for ordinary gzip (nothing to cut at), a bgzip file that is not whole BGZF blocks ending with the end-of-file block, a
+ * range with no unique guess, or a failed check: the results are then exactly f2q_submit_file's.
+ * f2q_get_info "shards" / "shard_fallback" on ctxs[0] tell how many contexts parsed the sample and whether it fell back.
+ */
+int f2q_submit_file_sharded(f2q_ctx** ctxs, int n, const char* path, int is_gzip, const uint64_t* cuts, int threads,
+                            int* complete, uint64_t* bytes_out);
+
 /* Same, but the chunk already lives in device memory of this context's GPU (resident mode).  The buffer
  * must stay valid and unmodified until the next f2q_end_sample/f2q_sync returns. */
 int f2q_submit_device(f2q_ctx* ctx, const void* dptr, uint64_t nbytes, int is_last);
@@ -312,7 +334,9 @@ int f2q_memo_counts(const f2q_ctx* ctx, uint64_t* lookups, uint64_t* hits);
  *   "seed_parts"    segments P of the resolver's seed plan; 0 = the classic m + 1 one-segment seeds (or no seed index)
  *   "flex_table"    1 when the library has the flex tables (every key <= 2 ACGT pieces of <= 32 symbols)
  *   "generic_reads" reads the generic read queue took during the last finished sample (one device-to-host copy per call;
- *                   F2Q_ESTATE inside a sample) */
+ *                   F2Q_ESTATE inside a sample)
+ *   "shards"        contexts that parsed the current / last sample (f2q_submit_file_sharded; 1 otherwise and after a fallback)
+ *   "shard_fallback" 1 when f2q_submit_file_sharded parsed the sample again on ctxs[0] alone */
 int f2q_get_info(f2q_ctx* ctx, const char* name, int64_t* value);
 
 /* device time of the last finished sample per kernel class, measured with CUDA events on the context's stream
