@@ -88,6 +88,7 @@ SYMBOLS = {
     "f2q_sequence_tinder": (C.c_int, [C.c_int, C.POINTER(Config), C.c_int32, C.c_char_p, C.c_uint32, C.c_char_p, C.c_uint32,
                                       _VP, _VP, _I32P, _I32P, _I32P]),
     "f2q_synth_fastq": (C.c_int, [_VP, C.POINTER(SynthSpec), _VP, _VP]),
+    "f2q_inflate_blocks": (C.c_int, [_VP, _VP, _VP, C.c_uint32, _VP, C.POINTER(C.c_uint32)]),
     "f2q_device_alloc": (C.c_int, [_VP, C.POINTER(_VP), C.c_uint64]),
     "f2q_device_free": (C.c_int, [_VP, _VP]),
     "f2q_memcpy_d2h": (C.c_int, [_VP, _VP, _VP, C.c_uint64]),
@@ -457,6 +458,16 @@ class Engine:
             return
         g = np.frombuffer(b"".join(guides), dtype=np.uint8)
         self._ck(self.L.f2q_synth_fastq(self.h, C.byref(s), g.ctypes.data, C.c_void_p(dptr)))
+
+    def inflate_blocks(self, d_comp: int, blocks, d_out: int) -> int:
+        """f2q_inflate_blocks: the bgzip inflate + CRC check of f2q_submit_file on len(blocks) payloads placed by the caller.
+        blocks: rows (src, csize, dst, isize, crc) (uint32; device offsets into d_comp / d_out).  Returns the device error
+        bits (0: every block inflated to its isize bytes with its CRC)."""
+        t = np.ascontiguousarray(np.asarray(blocks, dtype=np.uint32).reshape(-1, 5))
+        err = C.c_uint32(0)
+        self._ck(self.L.f2q_inflate_blocks(self.h, C.c_void_p(d_comp), t.ctypes.data if t.size else None, t.shape[0],
+                                           C.c_void_p(d_out), C.byref(err)))
+        return int(err.value)
 
     @property
     def launches(self) -> int:

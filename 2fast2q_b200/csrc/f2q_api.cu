@@ -120,7 +120,8 @@ struct f2q_ctx {
     DevBuf gz_comp[2], gz_out[2], gz_tab[2];
     BgzfBlock* gz_tab_host[2] = {nullptr, nullptr};
     cudaEvent_t gz_copied[2] = {nullptr, nullptr}, gz_free[2] = {nullptr, nullptr};
-    uint64_t gz_blocks = 0;                          // blocks inflated on the device by the last f2q_submit_file
+    uint64_t gz_blocks = 0;                          // non-empty blocks inflated on the device by the last file call (f2q_get_info)
+    uint64_t gz_batches = 0;                         // inflate launches of the last file call (f2q_get_info)
     FileRing* file_ring = nullptr;                   // page-locked ring of f2q_submit_file (allocated on first use)
     // multi-GPU (NCCL): the communicator this context is a rank of
     void* comm = nullptr; int comm_rank = 0, comm_size = 1; bool comm_owner = false;
@@ -1509,6 +1510,33 @@ namespace {
 constexpr size_t GZ_COMP_BYTES = 1u << 30, GZ_OUT_BYTES = 3ull << 30, GZ_MAX_BLOCKS = 1u << 16;
 const uint8_t BGZF_EOF[28] = {0x1f, 0x8b, 0x08, 0x04, 0, 0, 0, 0, 0, 0xff, 0x06, 0, 0x42, 0x43, 0x02, 0, 0x1b, 0, 0x03, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 
+// one batch of BGZF blocks (the table on the device), inflated on the context's stream and checked against their trailers:
+// the inflate kernel the options pick ("gpu_inflate" 1 lock-step lanes / 2 free-running threads, "gpu_inflate_bits"), then
+// k_bgzf_crc.  A block that is not valid DEFLATE data of its isize and CRC-32 sets ERR_INFLATE in *error.  The compressed
+// bytes must be readable 64 KiB past the last block, the output 16 bytes past it (aligned word loads)
+int inflate_launch(f2q_ctx* c, const uint8_t* comp, const BgzfBlock* tab, uint32_t nb, uint8_t* out, uint32_t* error) {
+    if (!nb) return F2Q_OK;
+    if (c->gpu_inflate_mode == 2)
+        k_inflate_bgzf<<<(nb + INFLATE_THREADS - 1) / INFLATE_THREADS, INFLATE_THREADS, 0, c->stream>>>(comp, tab, nb, out, error);
+    else {
+        const uint32_t grid = (nb + INFLATE_LANES - 1) / INFLATE_LANES;
+        if (!c->gz_attr) {
+            CU(c, cudaFuncSetAttribute(k_inflate_bgzf_lanes<9, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)inflate_smem<9, 7>()));
+            CU(c, cudaFuncSetAttribute(k_inflate_bgzf_lanes<8, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)inflate_smem<8, 6>()));
+            c->gz_attr = true;
+        }
+        // 9 + 7 index bits: 5 warps per SM; 8 + 6: 11 — the small tables when the batch can fill those warps
+        const bool small = c->gpu_inflate_bits ? c->gpu_inflate_bits == 8 : grid > 5u * (uint32_t)c->sm_count;
+        if (small) k_inflate_bgzf_lanes<8, 6><<<grid, INFLATE_LANES, inflate_smem<8, 6>(), c->stream>>>(comp, tab, nb, out, error);
+        else k_inflate_bgzf_lanes<9, 7><<<grid, INFLATE_LANES, inflate_smem<9, 7>(), c->stream>>>(comp, tab, nb, out, error);
+    }
+    k_bgzf_crc<<<(nb + CRC_WARPS - 1) / CRC_WARPS, CRC_WARPS * 32, 0, c->stream>>>(tab, nb, out, error);
+    c->launches += 2;
+    c->gz_batches++;
+    CU(c, cudaGetLastError());
+    return F2Q_OK;
+}
+
 // bgzip file -> the sample, inflated ON THE DEVICE: compressed pieces are read into the pinned ring, their block headers and
 // trailers are walked on the host (sizes only), the pieces go to a device staging buffer on the copy stream, and one launch
 // of k_inflate_bgzf_lanes per batch (<= 1 GiB compressed, <= 3 GiB of output, <= 65 536 blocks: tens of thousands of lanes) writes the FASTQ text straight
@@ -1548,8 +1576,10 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t begi
     bool eof = false, stop = false;
     int batch = 0;
     *finished = false;
-    c->gz_blocks = 0;
-    while (!eof && !stop) {
+    c->gz_blocks = 0; c->gz_batches = 0;
+    // a full batch ends the batch only: the blocks behind it are carried into the next one, also when the whole range has
+    // been read (eof).  Only a block cut off by the end of the range (or what is not a BGZF block) stops the device path
+    while (!(eof && carry.empty()) && !stop) {
         const int k = batch & 1;
         // batch k: the copy engine may overwrite its staging buffer only after the previous inflate out of it has finished
         CU(c, cudaStreamWaitEvent(c->copy_stream, c->gz_free[k], 0));
@@ -1558,10 +1588,11 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t begi
         double t0 = now();
         CU(c, cudaEventSynchronize(c->gz_free[k]));                    // (returns at once for an event that was never recorded)
         t_free += now() - t0;
-        uint32_t nb = 0;
+        uint32_t nb = 0, nonempty = 0;
         size_t comp_fill = 0, out_fill = 0;
         uint64_t batch_start = off - carry.size();
-        while (!eof && !stop && comp_fill + R.bytes + 65536 <= comp_target && out_fill + 4 * R.bytes <= out_cap && nb + 4096 < GZ_MAX_BLOCKS) {
+        bool full = false;
+        while (!(eof && carry.empty()) && !stop && !full && comp_fill + R.bytes + 65536 <= comp_target && out_fill + 4 * R.bytes <= out_cap && nb + 4096 < GZ_MAX_BLOCKS) {
             uint8_t* buf; int idx;
             t0 = now();
             if ((rc = ring_get(c, R, &buf, &idx))) return rc;
@@ -1586,19 +1617,23 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t begi
                 const uint32_t xlen = (uint32_t)(buf[p + 10] | buf[p + 11] << 8);
                 uint32_t isize; memcpy(&isize, buf + p + bs - 4, 4);
                 if (bs < 12u + xlen + 8u || isize > 65536u) { stop = true; break; }
-                if (out_fill + isize > out_cap || nb >= GZ_MAX_BLOCKS) break;
-                if (isize) { tab[nb++] = BgzfBlock{(uint32_t)(comp_fill + p + 12 + xlen), (uint32_t)(bs - 12 - xlen - 8), (uint32_t)out_fill, isize}; out_fill += isize; }
+                if (out_fill + isize > out_cap || nb >= GZ_MAX_BLOCKS) { full = true; break; }
+                // (empty blocks too: their payload and CRC are checked like every other block's)
+                uint32_t crc; memcpy(&crc, buf + p + bs - 8, 4);
+                tab[nb++] = BgzfBlock{(uint32_t)(comp_fill + p + 12 + xlen), (uint32_t)(bs - 12 - xlen - 8), (uint32_t)out_fill, isize, crc};
+                out_fill += isize; nonempty += isize != 0;
                 p += bs;
             }
             t_walk += now() - t0;
-            // copy the whole blocks to the device staging buffer; what is left (a partial block) is carried
+            // copy the whole blocks to the device staging buffer; what is left (a partial block, or the blocks behind a full
+            // batch) is carried
             if (p) CU(c, cudaMemcpyAsync(reinterpret_cast<uint8_t*>(c->gz_comp[k].p) + comp_fill, buf, p, cudaMemcpyHostToDevice, c->copy_stream));
             R.used[idx] = true;
             CU(c, cudaEventRecord(R.done[idx], c->copy_stream));
             comp_fill += p;
             if (stop) { off = batch_start + comp_fill; carry.clear(); break; }
             if (have > p) {
-                if (eof) { stop = true; off = off - (have - p); break; }    // a truncated last block: the host reader delivers its decodable part
+                if (eof && !full) { stop = true; off = off - (have - p); break; }    // a truncated last block: the host reader delivers its decodable part
                 carry.assign(buf + p, buf + have);
             }
             batch_start = off - carry.size() - comp_fill;
@@ -1609,36 +1644,14 @@ int submit_bgzf_gpu(f2q_ctx* c, FILE* f, FileRing& R, int threads, uint64_t begi
             CU(c, cudaEventRecord(c->gz_copied[k], c->copy_stream));
             CU(c, cudaStreamWaitEvent(c->stream, c->gz_copied[k], 0));
             // (the output buffer of batch k-2 was parsed by kernels earlier on this same stream)
-            if (c->gpu_inflate_mode == 2)
-                k_inflate_bgzf<<<(nb + INFLATE_THREADS - 1) / INFLATE_THREADS, INFLATE_THREADS, 0, c->stream>>>(
-                    reinterpret_cast<const uint8_t*>(c->gz_comp[k].p), reinterpret_cast<const BgzfBlock*>(c->gz_tab[k].p), nb,
-                    reinterpret_cast<uint8_t*>(c->gz_out[k].p), c->d_error);
-            else {
-                const uint32_t grid = (nb + INFLATE_LANES - 1) / INFLATE_LANES;
-                if (!c->gz_attr) {
-                    CU(c, cudaFuncSetAttribute(k_inflate_bgzf_lanes<9, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)inflate_smem<9, 7>()));
-                    CU(c, cudaFuncSetAttribute(k_inflate_bgzf_lanes<8, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)inflate_smem<8, 6>()));
-                    c->gz_attr = true;
-                }
-                // 9 + 7 index bits: 5 warps per SM; 8 + 6: 11 — the small tables when the batch can fill those warps
-                const bool small = c->gpu_inflate_bits ? c->gpu_inflate_bits == 8 : grid > 5u * (uint32_t)c->sm_count;
-                if (small)
-                    k_inflate_bgzf_lanes<8, 6><<<grid, INFLATE_LANES, inflate_smem<8, 6>(), c->stream>>>(
-                        reinterpret_cast<const uint8_t*>(c->gz_comp[k].p), reinterpret_cast<const BgzfBlock*>(c->gz_tab[k].p), nb,
-                        reinterpret_cast<uint8_t*>(c->gz_out[k].p), c->d_error);
-                else
-                    k_inflate_bgzf_lanes<9, 7><<<grid, INFLATE_LANES, inflate_smem<9, 7>(), c->stream>>>(
-                        reinterpret_cast<const uint8_t*>(c->gz_comp[k].p), reinterpret_cast<const BgzfBlock*>(c->gz_tab[k].p), nb,
-                        reinterpret_cast<uint8_t*>(c->gz_out[k].p), c->d_error);
-            }
-            c->launches++;
-            CU(c, cudaGetLastError());
+            if ((rc = inflate_launch(c, reinterpret_cast<const uint8_t*>(c->gz_comp[k].p), reinterpret_cast<const BgzfBlock*>(c->gz_tab[k].p), nb,
+                                     reinterpret_cast<uint8_t*>(c->gz_out[k].p), c->d_error))) return rc;
             CU(c, cudaEventRecord(c->gz_free[k], c->stream));
-            c->gz_blocks += nb;
+            c->gz_blocks += nonempty;
             *total += out_fill;
-            if ((rc = device_range(c, reinterpret_cast<const uint8_t*>(c->gz_out[k].p), out_fill, 0))) return rc;
+            if (out_fill && (rc = device_range(c, reinterpret_cast<const uint8_t*>(c->gz_out[k].p), out_fill, 0))) return rc;
             batch++;
-        } else if (!stop && !eof) return fail(c, F2Q_EINTERNAL, "bgzip batch without a block");
+        } else if (!stop && !(eof && carry.empty())) return fail(c, F2Q_EINTERNAL, "bgzip batch without a block");
     }
     if (debug) fprintf(stderr, "[f2q ingest] bgzf on the device: %d batches, %llu blocks; host thread: buffers %.1f ms, read %.1f ms, ring wait %.1f ms, batch wait %.1f ms, header walk %.1f ms\n",
                        batch, (unsigned long long)c->gz_blocks, t_alloc, t_read, t_ring, t_free, t_walk);
@@ -1662,6 +1675,7 @@ F2Q_EXPORT int f2q_submit_file(f2q_ctx* c, const char* path, int is_gzip, uint64
     setvbuf(f, nullptr, _IONBF, 0);
     if ((rc = ensure_ring(c))) { fclose(f); return rc; }
     FileRing& R = *c->file_ring;
+    c->gz_blocks = 0; c->gz_batches = 0;
     uint64_t total = 0, lines_left = limit_lines;
     bool stop = false;                                                 // preprocess mode: the line limit was reached
     // cut `n` bytes at the line limit; returns the bytes to submit
@@ -1748,7 +1762,7 @@ F2Q_EXPORT int f2q_submit_file(f2q_ctx* c, const char* path, int is_gzip, uint64
         }
     }
     if (bgzf) {
-        struct Blk { const uint8_t* src; uint32_t csize, isize; size_t dst; };
+        struct Blk { const uint8_t* src; uint32_t csize, isize, crc; size_t dst; };
         std::vector<Blk> blks;
         bool fell_back = false;
         while (!stop && !rc) {
@@ -1767,10 +1781,10 @@ F2Q_EXPORT int f2q_submit_file(f2q_ctx* c, const char* path, int is_gzip, uint64
                 const uint8_t* p = in.data() + in_pos;
                 const uint32_t xlen = (uint32_t)(p[10] | p[11] << 8);
                 if (bs < 12u + xlen + 8u) { corrupt = true; break; }
-                uint32_t isize; memcpy(&isize, p + bs - 4, 4);
+                uint32_t isize, crc; memcpy(&isize, p + bs - 4, 4); memcpy(&crc, p + bs - 8, 4);
                 if (isize > 65536u) { corrupt = true; break; }
                 if (out + isize > R.bytes + 65536) break;
-                blks.push_back({p + 12 + xlen, (uint32_t)(bs - 12 - xlen - 8), isize, out});
+                blks.push_back({p + 12 + xlen, (uint32_t)(bs - 12 - xlen - 8), isize, crc, out});
                 out += isize; in_pos += bs;
                 if (out >= R.bytes) break;
             }
@@ -1791,7 +1805,8 @@ F2Q_EXPORT int f2q_submit_file(f2q_ctx* c, const char* path, int is_gzip, uint64
                     z.next_in = const_cast<Bytef*>(blks[k].src); z.avail_in = blks[k].csize;
                     z.next_out = buf + blks[k].dst; z.avail_out = blks[k].isize;
                     const int zr = inflate(&z, Z_FINISH);
-                    if (zr != Z_STREAM_END || z.avail_out != 0) { bad[t] = 1; break; }
+                    // (raw deflate: the trailer's CRC-32 is checked here, as the serial reader's zlib does for every member)
+                    if (zr != Z_STREAM_END || z.avail_out != 0 || ::crc32(0, buf + blks[k].dst, blks[k].isize) != blks[k].crc) { bad[t] = 1; break; }
                 }
                 inflateEnd(&z);
             };
@@ -1905,7 +1920,7 @@ F2Q_EXPORT int f2q_end_sample(f2q_ctx* c, uint64_t* counts, uint64_t* stats) {
                 hs.dbg[0] >> 20, hs.dbg[7] >> 20, hs.dbg[1] >> 20, hs.dbg[4] >> 20, hs.dbg[2] >> 20, hs.dbg[3] >> 20, hs.dbg[5], hs.dbg[6] >> 20);
     if (err & ERR_RECORD_TOO_LONG) return fail(c, F2Q_ETOOLONG, "a FASTQ record is longer than carry_bytes; raise it with f2q_set_option");
     if (err & ERR_LOOKBACK_TIMEOUT) return fail(c, F2Q_EINTERNAL, "a device-side wait timed out; this sample's counts are invalid (the context stays usable)");
-    if (err & ERR_INFLATE) return fail(c, F2Q_EINVAL, "corrupted gzip data (a bgzip block did not inflate to its promised size on the device)");
+    if (err & ERR_INFLATE) return fail(c, F2Q_EINVAL, "corrupted gzip data (a bgzip block did not inflate to its promised size and CRC on the device)");
     if (err & ERR_EC_FULL) return fail(c, F2Q_EINTERNAL, "an Extract+Count table overflowed (a chunk whose line structure defeated the speculation held more keys than were reserved): rerun with option spec = 0");
     if (err) return fail(c, F2Q_EINTERNAL, "device-side failure, flags=" + std::to_string(err));
     if (counts && c->n_keys) CU(c, cudaMemcpy(counts, c->result.p, (size_t)c->n_keys * 8, cudaMemcpyDeviceToHost));
@@ -2721,6 +2736,8 @@ F2Q_EXPORT int f2q_get_info(f2q_ctx* c, const char* name, int64_t* value) {
     else if (n == "flex_table") *value = c->T.fx_slots ? 1 : 0;
     else if (n == "shards") *value = c->last_shards;
     else if (n == "shard_fallback") *value = c->last_shard_fallback;
+    else if (n == "gz_blocks") *value = (int64_t)c->gz_blocks;
+    else if (n == "gz_batches") *value = (int64_t)c->gz_batches;
     else if (n == "generic_reads") {
         if (c->in_sample) return fail(c, F2Q_ESTATE, "generic_reads is known once the sample has finished");
         unsigned long long v = 0;
@@ -2766,6 +2783,32 @@ F2Q_EXPORT int f2q_synth_fastq(f2q_ctx* c, const f2q_synth_spec* spec, const uin
     }
     CU(c, cudaGetLastError());
     if (guides) CU(c, cudaStreamSynchronize(c->stream));
+    return F2Q_OK;
+}
+
+// ---- the bgzip inflate of f2q_submit_file on blocks the caller placed (tests) ------------------------------------------
+F2Q_EXPORT int f2q_inflate_blocks(f2q_ctx* c, const void* d_comp, const uint32_t* blocks, uint32_t n, void* d_out, uint32_t* error_bits) {
+    int rc = check_ctx(c); if (rc) return rc;
+    if (c->in_sample) return fail(c, F2Q_ESTATE, "f2q_inflate_blocks inside a sample");
+    if (!error_bits || (n && (!d_comp || !blocks || !d_out))) return fail(c, F2Q_EINVAL, "null argument");
+    if (n > GZ_MAX_BLOCKS) return fail(c, F2Q_EINVAL, "f2q_inflate_blocks: more than 65536 blocks");
+    for (uint32_t b = 0; b < n; b++)
+        if (blocks[5 * (size_t)b + 3] > 65536u) return fail(c, F2Q_EINVAL, "f2q_inflate_blocks: a block of more than 64 KiB");
+    *error_bits = 0;
+    DevBuf tab;
+    if ((rc = dev_alloc(c, tab, (size_t)n * sizeof(BgzfBlock) + 16))) return rc;
+    uint32_t* d_err = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(tab.p) + (size_t)n * sizeof(BgzfBlock));
+    static_assert(sizeof(BgzfBlock) == 5 * sizeof(uint32_t), "f2q_inflate_blocks takes the block table as 5 words per block");
+    cudaError_t e = cudaMemsetAsync(d_err, 0, 4, c->stream);
+    if (e == cudaSuccess && n) e = cudaMemcpyAsync(tab.p, blocks, (size_t)n * sizeof(BgzfBlock), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) {
+        rc = inflate_launch(c, reinterpret_cast<const uint8_t*>(d_comp), reinterpret_cast<const BgzfBlock*>(tab.p), n, reinterpret_cast<uint8_t*>(d_out), d_err);
+        if (!rc) e = cudaMemcpyAsync(error_bits, d_err, 4, cudaMemcpyDeviceToHost, c->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    tab.release();
+    if (rc) return rc;
+    if (e != cudaSuccess) return fail(c, F2Q_ECUDA, std::string("f2q_inflate_blocks: ") + cudaGetErrorString(e));
     return F2Q_OK;
 }
 

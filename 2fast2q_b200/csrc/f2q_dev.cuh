@@ -19,7 +19,7 @@ constexpr uint32_t ERR_LOOKBACK_TIMEOUT = 1u;
 constexpr uint32_t ERR_RECORD_TOO_LONG = 2u;
 constexpr uint32_t ERR_QUEUE = 4u;
 constexpr uint32_t ERR_EC_FULL = 8u;
-constexpr uint32_t ERR_INFLATE = 16u;         // k_inflate_bgzf met a block that is not valid DEFLATE data of the promised size
+constexpr uint32_t ERR_INFLATE = 16u;         // a bgzip block is not valid DEFLATE data of the promised size and CRC-32
 
 // ------------------------------------------------------------------------------------------------
 // parameters

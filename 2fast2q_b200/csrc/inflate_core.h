@@ -10,7 +10,7 @@
 // the code lengths): small per-thread state (about 1 KB of local memory), no shared tables, and FASTQ text has short codes.
 // It is a pure function compiled for the device by nvcc and for the host by g++: tests/native/hostcheck.cpp checks it
 // against zlib on the CPU (stored, fixed and dynamic blocks, every compression level), the -m gpu tests against the same
-// files through the kernel.
+// files through the kernel.  The CRC-32 check of every inflated block (k_bgzf_crc) is at the end of this file.
 #pragma once
 
 #include <stdint.h>
@@ -271,11 +271,13 @@ F2Q_HD void infl_build_lut(const H& h, uint16_t* lut, uint32_t stride, int bits,
 }
 
 // 32 more input bits when there is room for them (words behind the stream's end read as what follows it in memory: a valid
-// stream never uses them, and the final check refuses a stream that did)
+// stream never uses them, and the final check refuses a stream that did).  A corrupted stream can ask for bits far behind its
+// end (up to 15 bits per output byte, or an endless chain of empty blocks): from 8 bytes behind the end it gets zeros, so that
+// no load leaves the 16 bytes of slack the caller provides
 F2Q_HD void infl_refill4(InflLane& L) {
     if (L.bitcnt <= 32u) {
         L.bitbuf |= (uint64_t)L.ahead << L.bitcnt; L.bitcnt += 32u; L.in_pos += 4u;
-        L.ahead = infl_word(L.in + L.in_pos);
+        L.ahead = L.in_pos <= L.in_len + 8u ? infl_word(L.in + L.in_pos) : 0u;
     }
 }
 F2Q_HD uint32_t infl_take(InflLane& L, uint32_t n) {
@@ -467,6 +469,66 @@ F2Q_HD int infl_lane_result(const InflLane& L) {
     if (L.out_pos != L.out_len) return 2;
     if ((uint64_t)L.in_pos * 8u - L.bitcnt > (uint64_t)L.in_len * 8u) return 1;
     return 0;
+}
+
+
+// ------------------------------------------------------------------------------------------------------------
+// CRC-32 of gzip (RFC 1952: reflected, polynomial 0xEDB88320, register preset and final value inverted): the trailer of
+// every BGZF block carries the CRC of its uncompressed bytes, and a corrupted Huffman stream usually still decodes to the
+// promised length, with wrong bytes.  The 32 lanes of a warp check one block: lane j hashes a contiguous slice with
+// slicing-by-4 tables, and the slices are joined by linearity,
+//     crc(A || B) = crc(A) * x^(8|B|) mod P  xor  crc(B),
+// so crc(block) = xor over lanes of crc(slice_j) * x^(8 * bytes behind slice_j) mod P.
+// ------------------------------------------------------------------------------------------------------------
+constexpr uint32_t CRC32_POLY = 0xEDB88320u;
+
+// entry i of the slicing-by-4 tables (4 x 256 words): table k, byte b = b followed by k zero bytes through the register
+F2Q_HD uint32_t crc32_table_entry(uint32_t i) {
+    uint32_t c = i & 255u;
+    const uint32_t rounds = 8u * ((i >> 8) + 1u);
+    for (uint32_t r = 0; r < rounds; r++) c = (c & 1u) ? (c >> 1) ^ CRC32_POLY : c >> 1;
+    return c;
+}
+
+// the register after n bytes at p (no inversion: crc32 = ~crc32_update(~0, ...)); aligned 32-bit words where it can
+F2Q_HD uint32_t crc32_update(uint32_t c, const uint8_t* p, uint32_t n, const uint32_t* tab) {
+    uint32_t i = 0;
+    for (; i < n && (reinterpret_cast<uintptr_t>(p + i) & 3u); i++) c = tab[(c ^ p[i]) & 255u] ^ (c >> 8);
+    for (; i + 4u <= n; i += 4u) {
+        c ^= infl_word(p + i);
+        c = tab[768u + (c & 255u)] ^ tab[512u + ((c >> 8) & 255u)] ^ tab[256u + ((c >> 16) & 255u)] ^ tab[c >> 24];
+    }
+    for (; i < n; i++) c = tab[(c ^ p[i]) & 255u] ^ (c >> 8);
+    return c;
+}
+
+// a * b mod P (bit 31 is x^0, as in the reflected register)
+F2Q_HD uint32_t crc32_mulmod(uint32_t a, uint32_t b) {
+    uint32_t p = 0;
+    for (int k = 0; k < 32; k++) {
+        if (a & (0x80000000u >> k)) p ^= b;
+        b = (b & 1u) ? (b >> 1) ^ CRC32_POLY : b >> 1;
+    }
+    return p;
+}
+
+// crc * x^(8n) mod P: the CRC of a prefix moved in front of n more bytes
+F2Q_HD uint32_t crc32_shift(uint32_t crc, uint32_t n) {
+    uint32_t sq = 1u << 23, p = 1u << 31;                              // x^8, 1
+    for (; n; n >>= 1) {
+        if (n & 1u) p = crc32_mulmod(sq, p);
+        sq = crc32_mulmod(sq, sq);
+    }
+    return crc32_mulmod(p, crc);
+}
+
+// lane `lane` of `lanes` (one CRC check of an n-byte block): the CRC of its slice, shifted over the bytes behind the slice.
+// The xor of all lanes' values is the block's CRC.  Slices are a multiple of 4 bytes long (word loads from the second on).
+F2Q_HD uint32_t crc32_lane_part(const uint8_t* p, uint32_t n, uint32_t lane, uint32_t lanes, const uint32_t* tab) {
+    const uint32_t s = ((n + lanes - 1u) / lanes + 3u) & ~3u;
+    const uint32_t beg = lane * s < n ? lane * s : n, end = beg + s < n ? beg + s : n;
+    if (beg == end) return 0u;
+    return crc32_shift(~crc32_update(~0u, p + beg, end - beg, tab), n - end);
 }
 
 }  // namespace f2q

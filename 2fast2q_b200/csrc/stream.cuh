@@ -180,7 +180,7 @@ __global__ void __launch_bounds__(256) k_shard_sum(unsigned long long* __restric
 // compressed sizes come from the headers and their output offsets from the trailers, so thousands decode at once straight
 // into the buffer the streaming kernel parses; only the COMPRESSED bytes cross PCIe.
 // ------------------------------------------------------------------------------------------------
-struct BgzfBlock { uint32_t src, csize, dst, isize; };
+struct BgzfBlock { uint32_t src, csize, dst, isize, crc; };      // (crc: the CRC-32 of the block's trailer)
 constexpr int INFLATE_THREADS = 64;
 
 // (first form: every lane follows its own control flow through inflate_raw — measured 1.01 active threads per warp instruction,
@@ -215,6 +215,22 @@ __global__ void __launch_bounds__(INFLATE_LANES) k_inflate_bgzf_lanes(const uint
     while (__any_sync(0xffffffffu, L.state != INFL_ST_DONE)) infl_step<LB, DB>(L, T, lut, dlut, INFLATE_LANES);
     infl_flush(L);
     if (b < n && infl_lane_result(L) != 0) atomicOr(error, ERR_INFLATE);
+}
+
+// behind either inflate kernel, on the same stream: the CRC-32 of every block's output against its trailer (inflate_core.h),
+// one warp per block, the slicing-by-4 tables in shared memory
+constexpr int CRC_WARPS = 8;
+__global__ void __launch_bounds__(CRC_WARPS * 32) k_bgzf_crc(const BgzfBlock* __restrict__ blk, uint32_t n, const uint8_t* __restrict__ out,
+                                                             uint32_t* error) {
+    __shared__ uint32_t tab[1024];
+    for (uint32_t i = threadIdx.x; i < 1024u; i += blockDim.x) tab[i] = crc32_table_entry(i);
+    __syncthreads();
+    const uint32_t b = blockIdx.x * CRC_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31u;
+    if (b >= n) return;                                                // (the whole warp)
+    const BgzfBlock B = blk[b];
+    uint32_t v = crc32_lane_part(out + B.dst, B.isize, lane, 32u, tab);
+    for (int d = 16; d; d >>= 1) v ^= __shfl_xor_sync(0xffffffffu, v, d);
+    if (lane == 0 && v != B.crc) atomicOr(error, ERR_INFLATE);
 }
 
 // start of a sample: result vector, scratch vector, error word and the stream state in ONE launch

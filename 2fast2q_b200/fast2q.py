@@ -480,7 +480,14 @@ def _count_file(raw, features, param, preprocess=False):
         except _lib.F2QError:
             pass
         raise
-    counts, stats = engine.end()
+    try:
+        counts, stats = engine.end()
+    except _lib.F2QError as e:
+        # a bgzip block inflated on the device that failed its size or CRC-32 check: reported when the sample ends
+        if e.code == -1 and "corrupted gzip" in str(e):
+            colourful_errors("WARNING", f"{raw} is an incomplete or corrupted gzip file. ({e})")
+            return None
+        raise
     if not complete:
         colourful_errors("WARNING", f"{raw} is an incomplete or corrupted gzip file. Only partial processing might have occurred.")
     return counts, stats, engine
@@ -927,7 +934,14 @@ def split_file_native(raw, features, param, devices):
     except BaseException:
         end_all()
         raise
-    counts, local_read_stats = engines[0].end()
+    try:
+        counts, local_read_stats = engines[0].end()
+    except _lib.F2QError as e:
+        end_all()
+        if e.code == -1 and "corrupted gzip" in str(e):     # (a bgzip block of some range failed its size or CRC-32 check)
+            colourful_errors("WARNING", f"{raw} is an incomplete or corrupted gzip file. ({e})")
+            return
+        raise
     for e in engines[1:]:
         e.end()                                              # (closed and empty: leaves the cached engine reusable)
     if not complete:

@@ -304,6 +304,16 @@ typedef struct f2q_synth_spec {
  * table uploaded by the previous call (per-chunk generation of workloads larger than HBM). */
 int f2q_synth_fastq(f2q_ctx* ctx, const f2q_synth_spec* spec, const uint8_t* guides, void* dptr);
 
+/* ---- the bgzip inflate of f2q_submit_file on blocks the caller placed (tests) -----------------
+ * Inflates n <= 65536 raw DEFLATE payloads with the kernels and the kernel choice f2q_submit_file uses for bgzip input
+ * (options "gpu_inflate" 1 lock-step / 2 free-running and "gpu_inflate_bits" 0 auto / 8 / 9), then checks every output
+ * against its CRC-32.  blocks = n x {src, csize, dst, isize, crc} on the HOST: block b's payload is d_comp[src, src + csize),
+ * its output goes to d_out[dst, dst + isize) (isize <= 65536), crc is the CRC-32 its output must have.  d_comp must be
+ * readable 64 KiB past the last payload and d_out 16 bytes past the last output, as the staging buffers are.
+ * *error_bits = 0 when every block inflated to exactly its isize bytes with its CRC, else the device error flags
+ * (ERR_INFLATE = 16).  Synchronous; F2Q_ESTATE inside a sample. */
+int f2q_inflate_blocks(f2q_ctx* ctx, const void* d_comp, const uint32_t* blocks, uint32_t n, void* d_out, uint32_t* error_bits);
+
 /* device memory helpers so that a non-CUDA host language can hold resident chunks */
 int f2q_device_alloc(f2q_ctx* ctx, void** dptr, uint64_t nbytes);
 int f2q_device_free(f2q_ctx* ctx, void* dptr);
@@ -336,7 +346,10 @@ int f2q_memo_counts(const f2q_ctx* ctx, uint64_t* lookups, uint64_t* hits);
  *   "generic_reads" reads the generic read queue took during the last finished sample (one device-to-host copy per call;
  *                   F2Q_ESTATE inside a sample)
  *   "shards"        contexts that parsed the current / last sample (f2q_submit_file_sharded; 1 otherwise and after a fallback)
- *   "shard_fallback" 1 when f2q_submit_file_sharded parsed the sample again on ctxs[0] alone */
+ *   "shard_fallback" 1 when f2q_submit_file_sharded parsed the sample again on ctxs[0] alone
+ *   "gz_blocks"     non-empty bgzip blocks inflated on the device by the last file call of this context (f2q_submit_file, or
+ *                   this context's range of f2q_submit_file_sharded); 0 when the host inflated them
+ *   "gz_batches"    inflate launches of that call (one batch: <= 65 536 blocks, <= the output buffer) */
 int f2q_get_info(f2q_ctx* ctx, const char* name, int64_t* value);
 
 /* device time of the last finished sample per kernel class, measured with CUDA events on the context's stream

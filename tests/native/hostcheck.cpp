@@ -112,6 +112,68 @@ __attribute__((visibility("default")))
 int hc_inflate_lane8(const uint8_t* in, uint32_t in_len, uint8_t* out, uint32_t out_len) { return inflate_lane<8, 6>(in, in_len, out, out_len); }
 }
 
+// ---- how far behind its input the lock-step decoder reads ----------------------------------------------------------------
+// The input ends 16 bytes before an inaccessible page (the slack inflate_core.h asks for); a load behind that is caught
+// (SIGSEGV -> siglongjmp) and reported as 99 instead of ending the process.
+#include <setjmp.h>
+#include <signal.h>
+#include <sys/mman.h>
+#include <unistd.h>
+
+static sigjmp_buf g_guard_jmp;
+static void guard_handler(int) { siglongjmp(g_guard_jmp, 1); }
+
+extern "C" __attribute__((visibility("default")))
+int hc_inflate_lane_guarded(const uint8_t* in, uint32_t in_len, uint32_t out_len) {
+    const size_t page = (size_t)sysconf(_SC_PAGESIZE), span = ((size_t)in_len + 16 + page - 1) / page * page;
+    uint8_t* m = static_cast<uint8_t*>(mmap(nullptr, span + page, PROT_READ | PROT_WRITE, MAP_PRIVATE | MAP_ANONYMOUS, -1, 0));
+    if (m == MAP_FAILED) return -1;
+    mprotect(m + span, page, PROT_NONE);
+    uint8_t* ip = m + span - 16 - in_len;                              // (alignment: whatever in_len gives)
+    memcpy(ip, in, in_len);
+    memset(ip + in_len, 0x5c, 16);
+    std::vector<uint8_t> obuf((size_t)out_len + 64, 0);
+    static thread_local uint16_t lut[1 << 9], dlut[1 << 7];
+    struct sigaction sa, old;
+    memset(&sa, 0, sizeof(sa)); sa.sa_handler = guard_handler; sigemptyset(&sa.sa_mask);
+    sigaction(SIGSEGV, &sa, &old);
+    volatile int rc = 99;
+    if (sigsetjmp(g_guard_jmp, 1) == 0) {
+        f2q::InflLane L;
+        f2q::InflTables T;
+        f2q::infl_lane_init(L, ip, in_len, obuf.data() + 16, out_len);
+        for (uint64_t it = 0; L.state != f2q::INFL_ST_DONE && it < (1ull << 26); it++) f2q::infl_step<9, 7>(L, T, lut, dlut, 1);
+        f2q::infl_flush(L);
+        rc = L.state == f2q::INFL_ST_DONE ? f2q::infl_lane_result(L) : 9;
+    }
+    sigaction(SIGSEGV, &old, nullptr);
+    munmap(m, span + page);
+    return rc;
+}
+
+// ---- the CRC-32 check of k_bgzf_crc, against zlib.crc32 ----------------------------------------------------------------
+static const uint32_t* crc_tables() {
+    static uint32_t tab[1024];
+    static bool ready = false;
+    if (!ready) { for (uint32_t i = 0; i < 1024; i++) tab[i] = f2q::crc32_table_entry(i); ready = true; }
+    return tab;
+}
+extern "C" {
+// the CRC of p[0, n) in one pass
+__attribute__((visibility("default")))
+uint32_t hc_crc32(const uint8_t* p, uint32_t n) { return ~f2q::crc32_update(~0u, p, n, crc_tables()); }
+// the CRC of p[0, n) as one warp of k_bgzf_crc computes it: the xor of `lanes` slice values
+__attribute__((visibility("default")))
+uint32_t hc_crc32_lanes(const uint8_t* p, uint32_t n, uint32_t lanes) {
+    uint32_t v = 0;
+    for (uint32_t j = 0; j < lanes; j++) v ^= f2q::crc32_lane_part(p, n, j, lanes, crc_tables());
+    return v;
+}
+// crc * x^(8n) mod P
+__attribute__((visibility("default")))
+uint32_t hc_crc32_shift(uint32_t crc, uint32_t n) { return f2q::crc32_shift(crc, n); }
+}
+
 // developer statistics: iterations of the lock-step machine by state (HEADER, SYMBOL, COPY, STORED)
 extern "C" __attribute__((visibility("default")))
 int hc_inflate_lane_stats(const uint8_t* in, uint32_t in_len, uint8_t* out, uint32_t out_len, uint64_t* stats) {

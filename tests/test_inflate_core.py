@@ -78,3 +78,85 @@ def test_corrupted_and_truncated_streams_are_refused():
             bad += 1
         assert rc != 0 or len(out) == len(data)
     assert bad > 150                                         # (a flipped bit may leave a valid stream of the same length; that is what the CRC is for)
+
+
+def test_corrupted_streams_read_no_further_than_the_slack():
+    """the lock-step decoder may read 16 bytes behind its input (the staging buffer's slack), never more, whatever the stream
+    asks for: a truncated stream whose output is far from complete, garbage, and streams of empty blocks"""
+    H = hostcheck.lib()
+    H.hc_inflate_lane_guarded.argtypes = [C.c_char_p, C.c_uint32, C.c_uint32]
+    data = next(d for n, d in payloads() if n == "fastq")
+    rnd = random.Random(12)
+    streams = [(raw_deflate(data, 6), len(data)), (raw_deflate(data, 1, zlib.Z_HUFFMAN_ONLY), len(data))]
+    for comp, n in list(streams):
+        for cut in (1, 2, 5, 17, 100, len(comp) // 3):
+            streams.append((comp[:cut], n))
+    streams += [(bytes(rnd.randrange(256) for _ in range(k)), 65536) for k in (1, 3, 8, 64, 500)]
+    streams += [(b"\x00\x00\x00\xff\xff" * 7, 65536), (b"\x02\x00" * 9, 100), (b"\x00" * 13, 65536)]
+    for k, (comp, n) in enumerate(streams):
+        rc = H.hc_inflate_lane_guarded(comp, len(comp), n)
+        assert rc != 99, (k, len(comp))                              # a load behind the slack
+        assert rc != 0 or k < 2, k
+    assert H.hc_inflate_lane_guarded(streams[0][0], len(streams[0][0]), len(data)) == 0
+
+
+def _crc_fns():
+    H = hostcheck.lib()
+    H.hc_crc32.restype = H.hc_crc32_lanes.restype = H.hc_crc32_shift.restype = C.c_uint32
+    H.hc_crc32.argtypes = [C.c_void_p, C.c_uint32]
+    H.hc_crc32_lanes.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32]
+    H.hc_crc32_shift.argtypes = [C.c_uint32, C.c_uint32]
+    return H
+
+
+def _at(data: bytes, align: int):
+    """data at an address with (address mod 8) == align; the buffer stays alive with the returned pointer"""
+    buf = C.create_string_buffer(len(data) + 16)
+    base = C.addressof(buf)
+    off = (align - base) % 8
+    C.memmove(base + off, data, len(data))
+    return buf, base + off
+
+
+def test_crc32_equals_zlib_at_every_length_and_alignment():
+    """the CRC-32 the device checks every inflated BGZF block with (crc32_update / crc32_lane_part, inflate_core.h): every
+    length 0-300 and random lengths up to 65 536, at start addresses 0-7 mod 8, in one pass and as a warp of 32 lanes
+    (and of 1, 3 and 7 lanes, so that slices of every length and position occur)"""
+    H = _crc_fns()
+    rnd = random.Random(21)
+    blob = bytes(rnd.randrange(256) for _ in range(65536 + 8))
+    lengths = list(range(301)) + [rnd.randrange(301, 65537) for _ in range(60)] + [65280, 65535, 65536]
+    for n in lengths:
+        data = blob[n % 7:n % 7 + n]
+        want = zlib.crc32(data) & 0xFFFFFFFF
+        for align in range(8):
+            keep, p = _at(data, align)
+            assert H.hc_crc32(p, n) == want, (n, align)
+            assert H.hc_crc32_lanes(p, n, 32) == want, (n, align)
+        for lanes in (1, 3, 7):
+            keep, p = _at(data, n % 8)
+            assert H.hc_crc32_lanes(p, n, lanes) == want, (n, lanes)
+    # a wrong byte anywhere changes the lanes' CRC
+    data = bytearray(blob[:65280])
+    keep, p = _at(bytes(data), 3)
+    good = H.hc_crc32_lanes(p, len(data), 32)
+    for pos in (0, 1, 2039, 2040, 2041, 32639, 65279):
+        bad = bytearray(data)
+        bad[pos] ^= 1 << rnd.randrange(8)
+        keep, p = _at(bytes(bad), 3)
+        assert H.hc_crc32_lanes(p, len(bad), 32) != good, pos
+
+
+def test_crc32_combine_at_random_split_points():
+    """crc(A || B) = shift(crc(A), |B|) xor crc(B), the operator that joins the lanes' slices"""
+    H = _crc_fns()
+    rnd = random.Random(22)
+    blob = bytes(rnd.randrange(256) for _ in range(70000))
+    for _ in range(300):
+        n = rnd.choice((rnd.randrange(0, 64), rnd.randrange(0, 65537)))
+        k = rnd.randrange(0, n + 1)
+        a, b = blob[:k], blob[k:n]
+        want = zlib.crc32(a + b) & 0xFFFFFFFF
+        assert H.hc_crc32_shift(zlib.crc32(a), len(b)) ^ (zlib.crc32(b) & 0xFFFFFFFF) == want, (n, k)
+    assert H.hc_crc32_shift(0x12345678, 0) == 0x12345678
+    assert H.hc_crc32_shift(0, 1000) == 0
